@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the rasterize -> sample -> approximate-gradient hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2] [--dump-outputs DIR]
 
 One "step" = one forward + backward of ``rasterize_rgba`` over one batch of synthetic views
 (BASELINE.json config 2: teapot, a batch of 64 views, 512x512, no anti-aliasing, RGBA with a
@@ -226,6 +226,26 @@ class ClockSampler(threading.Thread):
                 "reasons": sorted(self.reasons), "samples": len(s)}
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor of `arrays` as out_dir/<name>.npy in float32, DUMP_BYTES in all.  The smallest go
+    first, whole; a tensor larger than its share of what is left is written as a sample of its flattened
+    elements: ascending indices drawn by a generator seeded with 0, so runs with the same arguments write the
+    same elements and two builds can be compared element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel())):
+        a = t.detach().float()
+        share = (left // (len(arrays) - i) - 4096) // 4     # elements; 4 KB for the .npy header
+        if a.numel() > share:
+            idx = np.unique(np.random.default_rng(0).integers(0, a.numel(), size=share))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+        left -= a.numel() * 4 + 4096
+
+
 def physical_gpu_index(local):
     vis = os.environ.get("CUDA_VISIBLE_DEVICES")
     if vis:
@@ -309,10 +329,13 @@ def run_ours(args):
     shared = bool(w.get("shared"))
     if shared:
         leaves_host = [inp["v_world"][None].contiguous()]
+        leaf_names = ["vertices_world"]
     elif w.get("renderer"):
         leaves_host = [inp["v_world"][None].repeat(B, 1, 1).contiguous(), inp["textures"]]
+        leaf_names = ["vertices_world", "textures"]
     else:
         leaves_host = [inp["vertices"].cpu()] + ([inp["textures"]] if rgb else [])
+        leaf_names = ["vertices"] + (["textures"] if rgb else [])
     sizes = [t.numel() for t in leaves_host]
     offs = [sum(sizes[:i]) for i in range(len(sizes))]
     flat_in = torch.empty(sum(sizes), dtype=torch.float32, device=dev)
@@ -419,7 +442,7 @@ def run_ours(args):
     e0.record()
     t_host0 = time.perf_counter()
     for i in range(args.steps):
-        run_step()
+        images = run_step()
     host_ms = (time.perf_counter() - t_host0) * 1e3 / args.steps
     e1.record()
     # (no NVML call from this thread while it still has launches to issue: one query can take milliseconds, and a
@@ -437,6 +460,11 @@ def run_ours(args):
     ms_step = ms_total / args.steps
     total_views = V if scaling == "strong" else B * world
     value = total_views * S * S / 1e6 / (ms_step / 1e3)
+    # before anything else runs a step: the captured step's outputs are overwritten by the next one
+    if args.dump_outputs and rank == 0:
+        outputs = {"images": images}
+        outputs.update(("grad_" + n, p_.grad) for n, p_ in zip(leaf_names, params))
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- per-kernel pass (same inputs, right after the timed region): roofline numbers
     L.nr_profile_enable(1)
@@ -797,7 +825,16 @@ def main():
                     help="cfg3 study only: leave the gradient of the shared mesh un-reduced (isolates the cost of the exchange)")
     ap.add_argument("--unfused-camera", action="store_true", help="cfg2r: camera transform as torch ops")
     ap.add_argument("--eager", action="store_true", help="launch every step from Python instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (the images and the gradient of "
+                         "every differentiable input; rank 0's views) as DIR/<name>.npy, float32, at most 64 MB "
+                         "in all: a larger output is written as a fixed seeded sample of its elements")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm sizes its batch from a timing, so its "
+                 "outputs differ from run to run")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -10,7 +10,8 @@
  *   (1) the same two operators with the same argument meaning (nr_face_index_map_forward_safe,
  *       nr_compute_weight_map), and
  *   (2) the fused forward / backward of the whole path that rasterize_core drives
- *       (nr_rasterize_forward, nr_rasterize_backward, nr_differentiation_backward).
+ *       (nr_rasterize_forward, nr_rasterize_backward, nr_rasterize_backward_lights,
+ *       nr_differentiation_backward).
  *
  * Conventions
  *   - every pointer is a DEVICE pointer unless its name ends in _host; plain pointers and
@@ -251,6 +252,28 @@ NR_API int nr_rasterize_backward(const nrRasterConfig *cfg, const float *vertice
                           const float *grad_images, float *grad_vertices, float *grad_textures,
                           float *grad_vertices_textures, void *deterministic_scratch, const nrLights *lights,
                           void *stream);
+
+/*
+ * nr_rasterize_backward plus the gradient with respect to the light data (autograd of rasterize.py:256-283
+ * with respect to each light's color, direction and alpha).  nr_rasterize_backward is this call with
+ * grad_light_data = light_deterministic_scratch = NULL.
+ *
+ *   grad_light_data     [L, B, 8] out, ACCUMULATED into, in the layout of nrLights.data: colour 0..2,
+ *                       direction 3..5 (directional lights only), alpha 6 (specular lights only); the other slots
+ *                       are left as they are.  NULL = not wanted (no extra work).  Only lit colour calls
+ *                       (NR_DRAW_RGB and lights->num_lights > 0) have a light gradient; otherwise it is left as is.
+ *   light_deterministic_scratch  only with NR_DETERMINISTIC and a non-NULL grad_light_data: L * B * 8 zero-filled
+ *                       int64 (8-byte aligned); the light gradient is then bit-identical from run to run too.
+ * The per-pixel terms are summed per warp in registers (a fixed order), so each warp of a tile adds at most one
+ * value per (light, parameter).
+ */
+NR_API int nr_rasterize_backward_lights(const nrRasterConfig *cfg, const float *vertices, const int32_t *faces,
+                                 const float *vertices_textures, const int32_t *faces_textures,
+                                 const float *textures, const int32_t *face_index_map,
+                                 const float *images_internal, const float *aux_map, const int32_t *tile_list,
+                                 const float *grad_images, float *grad_vertices, float *grad_textures,
+                                 float *grad_vertices_textures, void *deterministic_scratch, const nrLights *lights,
+                                 float *grad_light_data, void *light_deterministic_scratch, void *stream);
 
 /*
  * Differentiation.backward (differentiation.py:13-36) on channels-last tensors, as the

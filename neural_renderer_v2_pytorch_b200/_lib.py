@@ -32,7 +32,7 @@ NR_DENSE_RASTER = 512
 SYMBOLS = (
     "nr_abi_version", "nr_last_error", "nr_num_channels", "nr_event_create", "nr_event_destroy",
     "nr_event_synchronize", "nr_event_query", "nr_deterministic_scratch_bytes", "nr_workspace_bytes", "nr_rasterize_forward", "nr_rasterize_backward",
-    "nr_differentiation_backward", "nr_face_index_map_forward_safe", "nr_compute_weight_map",
+    "nr_rasterize_backward_lights", "nr_differentiation_backward", "nr_face_index_map_forward_safe", "nr_compute_weight_map",
     "nr_profile_enable", "nr_profile_collect", "nr_camera_partial_blocks", "nr_camera_forward",
     "nr_camera_backward", "nr_camera_exchange_bytes", "nr_camera_backward_shared_allreduce",
 )
@@ -124,6 +124,9 @@ def lib():
                                        ctypes.POINTER(Lights), vp]
     L.nr_rasterize_backward.restype = ctypes.c_int
     L.nr_rasterize_backward.argtypes = [ctypes.POINTER(RasterConfig)] + [vp] * 14 + [ctypes.POINTER(Lights), vp]
+    L.nr_rasterize_backward_lights.restype = ctypes.c_int
+    L.nr_rasterize_backward_lights.argtypes = ([ctypes.POINTER(RasterConfig)] + [vp] * 14 +
+                                               [ctypes.POINTER(Lights), vp, vp, vp])
     L.nr_deterministic_scratch_bytes.restype = ctypes.c_size_t
     L.nr_deterministic_scratch_bytes.argtypes = [ctypes.POINTER(RasterConfig)]
     L.nr_differentiation_backward.restype = ctypes.c_int

@@ -366,6 +366,19 @@ int nr_rasterize_backward(const nrRasterConfig *cfg, const float *vertices, cons
                           const float *grad_images, float *grad_vertices, float *grad_textures,
                           float *grad_vertices_textures, void *deterministic_scratch, const nrLights *lights,
                           void *stream_) {
+    return nr_rasterize_backward_lights(cfg, vertices, faces, vertices_textures, faces_textures, textures,
+                                        face_index_map, images_internal, aux_map, tile_list, grad_images,
+                                        grad_vertices, grad_textures, grad_vertices_textures, deterministic_scratch,
+                                        lights, nullptr, nullptr, stream_);
+}
+
+int nr_rasterize_backward_lights(const nrRasterConfig *cfg, const float *vertices, const int32_t *faces,
+                                 const float *vertices_textures, const int32_t *faces_textures,
+                                 const float *textures, const int32_t *face_index_map,
+                                 const float *images_internal, const float *aux_map, const int32_t *tile_list,
+                                 const float *grad_images, float *grad_vertices, float *grad_textures,
+                                 float *grad_vertices_textures, void *deterministic_scratch, const nrLights *lights,
+                                 float *grad_light_data, void *light_deterministic_scratch, void *stream_) {
     if (int rc = check_config(cfg)) return rc;
     const bool aa = cfg->flags & NR_ANTI_ALIASING, rgb = cfg->flags & NR_DRAW_RGB;
     if (!vertices || !face_index_map || !images_internal || !grad_images || !grad_vertices)
@@ -395,6 +408,9 @@ int nr_rasterize_backward(const nrRasterConfig *cfg, const float *vertices, cons
         a.lights = nr::LightArgs{lights->num_lights, lights->types, lights->data, lights->vertex_normals,
                                  lights->grad_vertex_normals, nullptr};
     }
+    // without lights (or without colour) the light gradient is zero: nothing to add
+    a.grad_light = a.lights.num > 0 ? grad_light_data : nullptr;
+    a.det_light = nullptr;
     a.det_verts = a.det_tex = a.det_vt = a.det_vn = nullptr;
     a.det_scale = 4294967296.f;     // 2^32: resolution 2.3e-10, |sum| < 2.1e9
     if (cfg->flags & NR_DETERMINISTIC) {
@@ -412,6 +428,12 @@ int nr_rasterize_backward(const nrRasterConfig *cfg, const float *vertices, cons
             p += (size_t)cfg->batch * cfg->num_tex_vertices * 2;
         }
         if (a.lights.grad_vnormals) a.det_vn = p;
+        if (a.grad_light) {
+            if (!light_deterministic_scratch || ((uintptr_t)light_deterministic_scratch & 7))
+                return fail(NR_ERR_INVALID_ARGUMENT,
+                            "NR_DETERMINISTIC with grad_light_data needs light_deterministic_scratch (8-byte aligned, zero-filled)");
+            a.det_light = (long long *)light_deterministic_scratch;
+        }
     }
     a.B = cfg->batch;
     a.nv = cfg->num_vertices;

@@ -197,9 +197,68 @@ __device__ __forceinline__ void accumulate(float *dst_f, long long *dst_i, Index
     }
 }
 
+// Gradient of the light data [L, B, 8] from one warp of one view b (autograd of rasterize.py:256-283 with respect
+// to color / direction / alpha).  n = interpolated normal (not renormalised), w = d loss / d colour weight of the
+// lane's pixel; lanes with on == false contribute nothing.  Per light (warp-uniform loop):
+//   ambient      d color = w
+//   directional  d color = w a,  d direction = -(w . color) gate n          (a, gate as in light_weights)
+//   specular     d color = w a^alpha,  d alpha = (w . color) a^alpha ln a for a > 0, else 0 (torch's pow backward)
+// The parameters of a light are summed over the warp by an xor butterfly (fixed order), then lane i adds parameter i:
+// at most 7 accumulations per (warp, light), never one per pixel.
+template <bool DET>
+__device__ __forceinline__ void light_param_grads(const BackwardArgs &a, int b, int lane, bool on, const float n[3],
+                                                  const float w[3]) {
+    const LightArgs &L = a.lights;
+    for (int l = 0; l < L.num; ++l) {
+        const int type = __ldg(L.types + l);
+        const int kind = type & 3;
+        const size_t o = ((size_t)l * a.B + b) * 8;
+        const float *d = L.data + o;
+        float p[7] = {w[0], w[1], w[2], 0.f, 0.f, 0.f, 0.f};    // ambient: d color = w
+        if (kind != 0) {
+            const float cr = __ldg(d), cg = __ldg(d + 1), cb = __ldg(d + 2);
+            float dir[3] = {0.f, 0.f, 1.f};
+            if (kind == 1) { dir[0] = __ldg(d + 3); dir[1] = __ldg(d + 4); dir[2] = __ldg(d + 5); }
+            const float raw = __fadd_rn(__fadd_rn(__fmul_rn(-dir[0], n[0]), __fmul_rn(-dir[1], n[1])), __fmul_rn(-dir[2], n[2]));
+            const bool backside = (type & 4) != 0;
+            const float av = backside ? fabsf(raw) : fmaxf(raw, 0.f);
+            const float gate = backside ? (raw > 0.f ? 1.f : (raw < 0.f ? -1.f : 0.f)) : (raw > 0.f ? 1.f : 0.f);
+            const float s = w[0] * cr + w[1] * cg + w[2] * cb;
+            float inten = av;
+            if (kind == 2) {
+                inten = powf(av, __ldg(d + 6));
+                p[6] = av > 0.f ? s * inten * logf(av) : 0.f;
+            } else {
+                p[3] = -s * gate * n[0]; p[4] = -s * gate * n[1]; p[5] = -s * gate * n[2];
+            }
+            p[0] = w[0] * inten; p[1] = w[1] * inten; p[2] = w[2] * inten;
+        }
+        if (!on) {
+#pragma unroll
+            for (int i = 0; i < 7; ++i) p[i] = 0.f;
+        }
+        // parameters this kind has: colour always, direction for directional, alpha for specular
+        const bool has_dir = kind == 1, has_alpha = kind == 2;
+#pragma unroll
+        for (int i = 0; i < 7; ++i) {
+            if ((i >= 3 && i < 6 && !has_dir) || (i == 6 && !has_alpha)) continue;
+#pragma unroll
+            for (int m = 16; m > 0; m >>= 1) p[i] += __shfl_xor_sync(0xffffffffu, p[i], m);
+        }
+        float v = p[0];
+#pragma unroll
+        for (int i = 1; i < 7; ++i)
+            if (lane == i) v = p[i];
+        const bool mine = lane < 3 || (lane < 6 && has_dir) || (lane == 6 && has_alpha);
+        if (mine && v != 0.f) accumulate<DET>(a.grad_light, a.det_light, o + lane, v, a.det_scale);
+    }
+}
+
 // AUX: the forward left the normalised weights (and, with colour, the texel coordinate) of every foreground pixel
 // in the aux map: nothing of that is re-derived here (9 scattered vertex loads and 12 IEEE divisions less per pixel).
-template <int CT, bool NEED_UV, bool DET, bool AUX>
+// LGRAD: also sum the gradient of the light data (lit variants, CT = 0, with a.grad_light); a variant of its own, so
+// that calls with constant lights run exactly the code they ran before light gradients existed.
+template <int CT, bool NEED_UV, bool DET, bool AUX, bool LGRAD = false>
 __global__ void __launch_bounds__(TILE_THREADS, 4)
 k_backward(const BackwardArgs a) {
     pdl_wait();         // the forward's maps, tile list and zero-filled accumulators (nr_kernels.h)
@@ -287,6 +346,10 @@ k_backward(const BackwardArgs a) {
     int tap[4] = {-1, -1, -1, -1};
     int cell = 0;
     bool has_tex = false;
+    // light-parameter gradients: the interpolated normal and d loss / d colour weight of a lit pixel, kept
+    // outside the divergent per-pixel code for the warp reduction at the end of the work item
+    bool lg_on = false;
+    float lg_n[3] = {0.f, 0.f, 0.f}, lg_w[3] = {0.f, 0.f, 0.f};
     // CT = 1 is a lone silhouette or depth channel, CT >= 3 always holds the three colour channels
     const bool rgb = (CT == 1) ? false : ((CT >= 3) ? true : (a.flags & FLAG_RGB) != 0);
     constexpr bool LIT = (CT == 0);      // lights only in the generic variants (keeps the common ones small)
@@ -375,6 +438,14 @@ k_backward(const BackwardArgs a) {
                             if (gn[c] != 0.f)
                                 accumulate<DET>(a.lights.grad_vnormals, a.det_vn, ovn + 3 * (size_t)vid[k] + c, q[k] * gn[c], a.det_scale);
                 }
+                if (LGRAD && lit) {
+                    lg_on = true;
+#pragma unroll
+                    for (int c = 0; c < 3; ++c) {
+                        lg_n[c] = nrm[c];
+                        lg_w[c] = g_lit[c] * rgb_tex[c];
+                    }
+                }
                 has_tex = true;
 #pragma unroll
                 for (int t = 0; t < 4; ++t)
@@ -455,6 +526,9 @@ k_backward(const BackwardArgs a) {
             }
         }
     }
+    // ---- light parameters: summed over the warp's 32 pixels, one accumulation per (warp, light, parameter)
+    if (LIT && LGRAD && __ballot_sync(0xffffffffu, lg_on) != 0u)
+        light_param_grads<DET>(a, b, lane, lg_on, lg_n, lg_w);
     }   // tiles
 }
 
@@ -490,7 +564,20 @@ cudaError_t launch_backward(const BackwardArgs &a, cudaStream_t stream) {
     const int grid = (int)(tiles < (long long)a.sm_count * 4 ? tiles : (long long)a.sm_count * 4);
     dim3 block(TILE_THREADS);
     ProfScope p(PROF_BACKWARD, stream);
-    if (a.det_verts) {
+    const long long px = (long long)a.B * a.R * a.R;
+    if (a.grad_light && a.lights.num > 0) {
+        // light gradients: the lit variants with the light-parameter reduction (a.C does not matter: CT = 0)
+        if (a.det_verts) {
+            if (a.grad_vt) launch_after(2, px, k_backward<0, true, true, false, true>, dim3(grid), block, 0, stream, a);
+            else launch_after(2, px, k_backward<0, false, true, false, true>, dim3(grid), block, 0, stream, a);
+        } else if (a.grad_vt) {
+            if (a.aux) launch_after(2, px, k_backward<0, true, false, true, true>, dim3(grid), block, 0, stream, a);
+            else launch_after(2, px, k_backward<0, true, false, false, true>, dim3(grid), block, 0, stream, a);
+        } else {
+            if (a.aux) launch_after(2, px, k_backward<0, false, false, true, true>, dim3(grid), block, 0, stream, a);
+            else launch_after(2, px, k_backward<0, false, false, false, true>, dim3(grid), block, 0, stream, a);
+        }
+    } else if (a.det_verts) {
         if (a.grad_vt) launch_after(2, (long long)a.B * a.R * a.R, k_backward<0, true, true, false>, dim3(grid), block, 0, stream, a);
         else launch_after(2, (long long)a.B * a.R * a.R, k_backward<0, false, true, false>, dim3(grid), block, 0, stream, a);
     } else if (a.grad_vt) {
@@ -522,6 +609,7 @@ cudaError_t launch_backward(const BackwardArgs &a, cudaStream_t stream) {
     conv(a.det_tex, a.grad_tex, (size_t)a.B * 3 * a.H * a.W);
     conv(a.det_vt, a.grad_vt, (size_t)a.B * a.nvt * 2);
     conv(a.det_vn, a.lights.grad_vnormals, (size_t)a.B * a.nv * 3);
+    conv(a.det_light, a.grad_light, (size_t)a.lights.num * a.B * 8);
     return cudaGetLastError();
 }
 

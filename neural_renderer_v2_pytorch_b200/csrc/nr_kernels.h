@@ -102,6 +102,10 @@ struct BackwardArgs {
     LightArgs lights;
     int B, nv, nf, R, S, ntx, C, flags, nvt, H, W;
     float eps;
+    // gradient of the light data [L, B, 8] (colour 0..2, direction 3..5, alpha 6), accumulated; null = none.
+    // Read by the lit variants only.  det_light: its fixed-point accumulator in deterministic mode.
+    float *grad_light;
+    long long *det_light;
 };
 cudaError_t launch_backward(const BackwardArgs &a, cudaStream_t stream);
 

@@ -317,19 +317,21 @@ def _validate_indices(idx, limit, what):
 
 
 class _Rasterize(torch.autograd.Function):
-    """Forward: nr_rasterize_forward. Backward: nr_rasterize_backward (Differentiation stencil +
-    every autograd edge the reference has on this path)."""
+    """Forward: nr_rasterize_forward. Backward: nr_rasterize_backward_lights (Differentiation stencil +
+    every autograd edge the reference has on this path, the light parameters included).  ``light_data`` is the
+    [L,B,8] tensor of lights.pack_lights, an input of its own so that autograd sees it; ``light_types`` its [L]
+    types."""
 
     @staticmethod
-    def forward(ctx, vertices, vertices_textures, textures, vertex_normals, backgrounds, faces, faces_textures, cfg,
-                light_pack):
+    def forward(ctx, vertices, vertices_textures, textures, vertex_normals, backgrounds, light_data, faces,
+                faces_textures, cfg, light_types):
         v = _f32c(vertices)
         bg = _f32c(backgrounds) if backgrounds is not None else None
         vt = _f32c(vertices_textures) if vertices_textures is not None else None
         tex = _f32c(textures) if textures is not None else None
         lights = None
-        if light_pack is not None:
-            lights = (light_pack[0], light_pack[1], _f32c(vertex_normals))
+        if light_data is not None:
+            lights = (light_types, _f32c(light_data), _f32c(vertex_normals))
         # The backward ADDS into its outputs.  When a backward is coming its accumulators are allocated
         # here and zero-filled by the raster kernel on the side (nrZeroFill) instead of by separate
         # fill kernels in front of the backward.
@@ -349,7 +351,8 @@ class _Rasterize(torch.autograd.Function):
         ctx.bg_dtype = backgrounds.dtype if backgrounds is not None else None
         ctx.has_tex = tex is not None
         ctx.has_lights = lights is not None
-        ctx.in_dtypes = tuple(t.dtype if t is not None else None for t in (vertices, vertices_textures, textures, vertex_normals))
+        ctx.in_dtypes = tuple(t.dtype if t is not None else None
+                              for t in (vertices, vertices_textures, textures, vertex_normals, light_data))
         ctx.has_aux = aux is not None
         saved = [v, faces, fim, internal if internal is not None else images, tile_list]
         if ctx.has_aux:
@@ -394,18 +397,22 @@ class _Rasterize(torch.autograd.Function):
             gvt = (pre[1] if pre[1] is not None else torch.zeros_like(vt)) if (need_vt and vt is not None) else None
             gtex = (pre[2] if pre[2] is not None else torch.zeros_like(tex)) if (need_tex and tex is not None) else None
             gvn = torch.zeros_like(lights[2]) if (lights is not None and ctx.needs_input_grad[3]) else None
-            scratch = None
+            # d loss / d light data [L,B,8] (colour, direction, alpha), summed by the backward kernel
+            glight = torch.zeros_like(lights[1]) if (lights is not None and ctx.needs_input_grad[5]) else None
+            scratch = lscratch = None
             if cfg.flags & _lib.NR_DETERMINISTIC:
                 scratch = torch.zeros(L.nr_deterministic_scratch_bytes(ctypes.byref(cfg)) // 8, dtype=torch.int64, device=dev)
-            rc = L.nr_rasterize_backward(ctypes.byref(cfg), _ptr(v), _ptr(faces), _ptr(vt), _ptr(ft),
-                                         _ptr(tex), _ptr(fim), _ptr(internal), _ptr(aux), _ptr(tile_list), _ptr(g), _ptr(gv),
-                                         _ptr(gtex), _ptr(gvt), _ptr(scratch), _lights_struct(lights, gvn),
-                                         ctypes.c_void_p(stream))
-            _lib.check(rc, "nr_rasterize_backward")
+                if glight is not None:
+                    lscratch = torch.zeros(glight.numel(), dtype=torch.int64, device=dev)
+            rc = L.nr_rasterize_backward_lights(ctypes.byref(cfg), _ptr(v), _ptr(faces), _ptr(vt), _ptr(ft),
+                                                _ptr(tex), _ptr(fim), _ptr(internal), _ptr(aux), _ptr(tile_list), _ptr(g),
+                                                _ptr(gv), _ptr(gtex), _ptr(gvt), _ptr(scratch), _lights_struct(lights, gvn),
+                                                _ptr(glight), _ptr(lscratch), ctypes.c_void_p(stream))
+            _lib.check(rc, "nr_rasterize_backward_lights")
         cast = lambda g_, dt: g_.to(dt) if (g_ is not None and dt is not None and g_.dtype != dt) else g_
-        dv, dvt, dtex, dvn = ctx.in_dtypes
+        dv, dvt, dtex, dvn, dlight = ctx.in_dtypes
         return ((cast(gv, dv) if need_v else None), cast(gvt, dvt), cast(gtex, dtex), cast(gvn, dvn), gbg,
-                None, None, None, None)
+                cast(glight, dlight), None, None, None, None)
 
 
 def _prepare(vertices, faces, params, hyperparams):
@@ -460,14 +467,15 @@ def _prepare(vertices, faces, params, hyperparams):
     if hyperparams.draw_rgb and params.lights is not None:      # an empty list renders black, rasterize.py:252-283
         # shading: per-vertex normals by differentiable torch ops (O(nv + nf)), the per-pixel part in the kernels
         light_pack = light_lib.pack_lights(params.lights, B, dev)
-        vn = light_lib.vertex_normals(vertices, faces_d)
+        vn = light_lib.vertex_normals(vertices, faces_d, deterministic=bool(cfg.flags & _lib.NR_DETERMINISTIC))
     return cfg, faces_d, vt, ft, tex, vn, light_pack, bg
 
 
 def rasterize_core(vertices, faces, params: RasterizeParam, hyperparams: RasterizeHyperparam):
     """``rasterize.py:194-329``. vertices [B,nv,3] screen space, faces [nf,3] -> images [B,C,S,S]."""
     cfg, faces_d, vt, ft, tex, vn, light_pack, bg = _prepare(vertices, faces, params, hyperparams)
-    return _Rasterize.apply(vertices, vt, tex, vn, bg, faces_d, ft, cfg, light_pack)
+    light_types, light_data = light_pack if light_pack is not None else (None, None)
+    return _Rasterize.apply(vertices, vt, tex, vn, bg, light_data, faces_d, ft, cfg, light_types)
 
 
 def rasterize_maps(vertices, faces, params: RasterizeParam, hyperparams: RasterizeHyperparam):
@@ -478,7 +486,7 @@ def rasterize_maps(vertices, faces, params: RasterizeParam, hyperparams: Rasteri
         images, internal, fim, wmap, dmap, _, _ = _forward_call(
             cfg, _f32c(vertices), faces_d, _f32c(vt) if vt is not None else None, ft,
             _f32c(tex) if tex is not None else None, True,
-            (light_pack[0], light_pack[1], _f32c(vn)) if light_pack is not None else None,
+            (light_pack[0], _f32c(light_pack[1]), _f32c(vn)) if light_pack is not None else None,
             _f32c(bg) if bg is not None else None)
     return dict(images=images, internal_images=internal if internal is not None else images,
                 face_index_map=fim, weight_map=wmap, depth_map=dmap)

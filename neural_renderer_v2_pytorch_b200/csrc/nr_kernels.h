@@ -1,5 +1,6 @@
 // nr_kernels.h -- internal launcher interfaces (not part of the C ABI).
 #pragma once
+#include <cuda.h>       // CUtensorMap (types only: the encoder is fetched through the runtime, no -lcuda)
 #include "nr_common.cuh"
 
 namespace nr {
@@ -106,6 +107,9 @@ struct BackwardArgs {
     // Read by the lit variants only.  det_light: its fixed-point accumulator in deterministic mode.
     float *grad_light;
     long long *det_light;
+    // Tensor maps of the staged front of k_backward (nr_backward.cu): face_index_map [B, R, R], the stencil image
+    // [B*C, R, R] and grad_images [B*C, S, S].  Filled by launch_backward; unused by the unstaged path.
+    CUtensorMap map_fim, map_img, map_grad;
 };
 cudaError_t launch_backward(const BackwardArgs &a, cudaStream_t stream);
 

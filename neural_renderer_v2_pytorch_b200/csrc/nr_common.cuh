@@ -13,7 +13,7 @@ namespace nr {
 
 constexpr int TILE = 16;            // tile edge in pixels (internal resolution)
 constexpr int TILE_THREADS = 256;   // one thread per pixel of a tile
-constexpr int WARP_BW = 8;          // a warp owns an 8 x 4 pixel block of the tile
+constexpr int WARP_BW = 8;          // a warp's 8 x 4 pixel block in tile_pixel() and shade_block()
 constexpr int WARP_BH = 4;
 
 // nrRasterConfig.flags (include/nr_b200.h)

@@ -54,15 +54,20 @@ __device__ __forceinline__ bool block_outside_face(float x0, float y0, float x1,
 }
 
 
-// Persistent kernel over the non-empty tiles.  The unit of work is one WARP = one 8x4 pixel block
-// of a tile, claimed with one atomicAdd (the next claim is in flight while the current block is
-// processed); the blocks of a tile are neighbours in the claim order, so its records are shared through
-// L1 / L2.  Warps never wait for each other: a block without candidate faces costs one cull pass.
+// Persistent kernel over the non-empty tiles.  The unit of work is one WARP = one 8x8 pixel block
+// of a tile, two pixels per lane: lane l owns (l & 7, l >> 3) of the upper 8x4 half and the pixel four rows
+// below it in the lower half.  A block is claimed from a per-CTA cursor (see "Scheduling"); the blocks of a
+// tile are neighbours in the claim order, so its records are shared through L1 / L2.  Warps never wait for
+// each other: a block without candidate faces costs one cull pass.
 // Per 32 faces of the tile list: every lane loads one face record, tests its pixel box against the
 // block, the survivors are compacted (ballot) into this warp's slice of shared memory with their edge
-// deltas and their pixel box as a bit mask over the block, then evaluated per pixel in list order.
+// deltas and their pixel box as a bit mask over each half, then evaluated per pixel in list order.
+// Culling 8x8 blocks instead of 8x4 halves the cull, compaction and claim work per pixel; the edge
+// functions are still evaluated only for the faces whose box touches the pixel's half.
 // Every pixel of the block is written (background included), see "output initialisation" above.
 constexpr int RASTER_WARPS = TILE_THREADS / 32;
+constexpr int BLK = 8;          // a warp's block is BLK x BLK pixels, in two 8x4 halves
+constexpr int HALF_H = 4;
 
 // NR_LAZY_Z: the z-test of a REGULAR candidate (face_z_regular, weights_one_sign: nothing cancels) is decided
 // with fast_zp() whenever the outcome is clear of its error bound, which it is for everything but near-ties:
@@ -72,17 +77,38 @@ constexpr int RASTER_WARPS = TILE_THREADS / 32;
 #ifndef NR_LAZY_Z
 #define NR_LAZY_Z 1
 #endif
-// NR_CPASYNC_STAGE (experiment, profiles/r2_cpasync_ab.txt): the 48-byte record of the NEXT group's face goes
-// global -> shared with three cp.async (LDGSTS) per lane into a per-warp double buffer instead of three LDG.128
-// into registers.  The records a warp needs are a gather (tile list -> record), so a bulk-tensor TMA copy has
-// nothing contiguous to move; cp.async is the asynchronous copy that fits, and it was measured.
-#ifndef NR_CPASYNC_STAGE
-#define NR_CPASYNC_STAGE 0
-#endif
 constexpr int REC_Q = NR_LAZY_Z ? 5 : 4;       // float4 per staged face
 
 __device__ __noinline__ float exact_zp_call(float w0, float w1, float w2, float z0, float z1, float z2) {
     return exact_zp(w0, w1, w2, z0, z1, z2);
+}
+
+// z-buffer state of one pixel: the running minimum, whether it is the reference's exact value, the winner.
+// The winner's raw weights and corner depths are not carried: they are recomputed from its record
+// (winner_weights) where they are needed, with the same arithmetic on the same floats.
+struct ZPix {
+    float depth_min;
+    bool dexact;
+    int best;
+};
+
+// raw weight numerators at (xp, yp) and corner depths of face f (its record, rasterize_cuda_kernel.cu:129-132)
+__device__ __forceinline__ void winner_weights(const FaceRec *rec_b, int f, float xp, float yp, float &w0, float &w1,
+                                               float &w2, float &z0, float &z1, float &z2) {
+    const float4 *rp = reinterpret_cast<const float4 *>(rec_b + f);
+    const float4 q0 = __ldg(rp), q1 = __ldg(rp + 1);
+    z2 = __ldg(reinterpret_cast<const float *>(rp + 2));
+    raw_weights(xp, yp, q0.x, q0.y, q0.w, q1.x, q1.z, q1.w, w0, w1, w2);
+    z0 = q0.z;
+    z1 = q1.y;
+}
+
+// the reference's inside test (rasterize_cuda_kernel.cu:107-116) against a staged face
+__device__ __forceinline__ bool edge_inside(float xp, float yp, const float4 &A, const float4 &Bq, const float4 &Cq) {
+    const float c1 = __fmaf_rn(__fsub_rn(yp, A.y), Bq.z, -__fmul_rn(Bq.w, __fsub_rn(xp, A.x)));
+    const float c2 = __fmaf_rn(__fsub_rn(yp, A.w), Cq.x, -__fmul_rn(Cq.y, __fsub_rn(xp, A.z)));
+    const float c3 = __fmaf_rn(__fsub_rn(yp, Bq.y), Cq.z, -__fmul_rn(Cq.w, __fsub_rn(xp, Bq.x)));
+    return !((__fmul_rn(c1, c2) < 0.f) | (__fmul_rn(c2, c3) < 0.f));
 }
 
 // Variants: RGB (texture sampling), AA (2x2 mean epilogue), FULL (everything optional: lights,
@@ -94,13 +120,9 @@ __global__ void __launch_bounds__(TILE_THREADS, 4)
 k_raster(const RasterArgs a) {
     pdl_wait();         // the binning kernel's records, lists and header (nr_kernels.h)
     pdl_trigger();      // the backward may be scheduled as this kernel's CTAs leave
-    // a tile is 16x16 pixels = 8 warp blocks (8x4 each), or in the FINE variants 8x8 = 2 blocks
-    constexpr int TSZ = FINE ? FINE_TILE : TILE, BLK_SHIFT = FINE ? 1 : 3, BLKS = 1 << BLK_SHIFT;
+    constexpr int TSZ = FINE ? FINE_TILE : TILE;
     __shared__ float4 s_rec[RASTER_WARPS][32][REC_Q];
-#if NR_CPASYNC_STAGE
-    __shared__ float4 s_stage[RASTER_WARPS][2][32][3];
-#endif
-    __shared__ uint32_t s_bb[RASTER_WARPS][32];
+    __shared__ uint2 s_bb[RASTER_WARPS][32];
 
     // If the pair list did not fit the workspace, the lists are unusable: every block then scans ALL
     // faces of its view (the records are complete regardless), which is the reference's own loop with
@@ -109,14 +131,18 @@ k_raster(const RasterArgs a) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int R = a.R;
     const TileList tl = open_tile_list(a.tile_list, a.B * a.ntx * a.ntx);
-    const int items = tl.total * BLKS;
-    constexpr bool aa = AA;
+    // A tile is 16x16 pixels = 4 warp blocks of 8x8, or in the FINE variants 8x8 = 1 block.  When even the
+    // 8x4 blocks of all tiles fit in one wave of resident warps (e.g. a single view), the kernel is bound by
+    // the latency of its slowest block, not by issue: it then runs 8x4 blocks (the lower pixel of a lane
+    // idles), 8 per 16x16 tile or 2 per 8x8 tile, and a warp has half the pixels to walk in series.
+    const bool tall = (long long)tl.total * (FINE ? 2 : 8) > (long long)a.sm_count * 4 * RASTER_WARPS;
+    const int bh = tall ? BLK : HALF_H;                                   // block height
+    const int blk_shift = (FINE ? 0 : 2) + (tall ? 0 : 1), items = tl.total << blk_shift;
     const bool has_bg = FULL && RGB && a.lights.backgrounds != nullptr;
-    const bool pow2 = (R & (R - 1)) == 0;
-    const float invR = 1.f / (float)R;          // exact for power-of-two R
+    const PixGrid grid(R);
     const unsigned lt_mask = (1u << lane) - 1u;
     float4 (*my_rec)[REC_Q] = s_rec[wid];
-    uint32_t *my_bb = s_bb[wid];
+    uint2 *my_bb = s_bb[wid];
 
     // ---- fill items (stores only, nr_shade.cuh), interleaved with the raster items: claim i also performs
     // fill item i (a static share per warp was slower: the warps holding the heavy tiles kept their fills
@@ -124,7 +150,7 @@ k_raster(const RasterArgs a) {
     const FillPlan plan = make_fill_plan(a);
     const int fill_items = plan.fill_items;
 
-    // Scheduling: the CTA claims EIGHT consecutive items (the blocks of one 16x16 tile) with one global
+    // Scheduling: the CTA claims EIGHT consecutive items (the blocks of two 16x16 tiles, of one with 8x4 blocks) with one global
     // atomicAdd and its warps take them one by one from a shared cursor, so the blocks of a tile run on the
     // same SM at about the same time (face records and lists shared through L1) and no warp waits for
     // another except while a batch is being fetched.  One shared word holds both the batch and the number
@@ -157,73 +183,42 @@ k_raster(const RasterArgs a) {
         if (first >= all_items) break;
         if (first < fill_items) do_fill_item<AA, FULL, FINE>(a, plan, first, lane);
     for (int item = first; item < min(first + GRAB, items); ++item) {
-        const int4 e0 = tile_entry(tl, item >> BLK_SHIFT);
-        const int sub = item & (BLKS - 1);
+        const int4 e0 = tile_entry(tl, item >> blk_shift);
+        const int sub = item & ((1 << blk_shift) - 1);
         const int b = e0.x, n = overflow ? a.nf : e0.w;
         const int32_t *list = a.pairs + e0.z;
-        const int wx0 = (e0.y & 0xffff) * TSZ + (FINE ? 0 : (sub & 1) * WARP_BW), wx1 = wx0 + WARP_BW - 1;
-        const int wy0 = (e0.y >> 16) * TSZ + (FINE ? sub : (sub >> 1)) * WARP_BH, wy1 = wy0 + WARP_BH - 1;
+        const int wx0 = (e0.y & 0xffff) * TSZ + (FINE ? 0 : (sub & 1) * BLK), wx1 = wx0 + BLK - 1;
+        const int wy0 = (e0.y >> 16) * TSZ + (FINE ? sub : (sub >> 1)) * bh, wy1 = wy0 + bh - 1;
+        // this lane's pixels: (xi, yi) in the upper half, (xi, yi + HALF_H) in the lower one
         const int xi = wx0 + (lane & 7), yi = wy0 + (lane >> 3);
-        const bool valid = (xi < R) && (yi < R);
-        const float xp = pow2 ? __fmul_rn((float)(2 * xi + 1 - R), invR) : pix_center(xi, R);
-        const float yp = pow2 ? __fmul_rn((float)(2 * yi + 1 - R), invR) : pix_center(yi, R);
+        const float xp = grid.center(xi);
+        const float yp_u = grid.center(yi), yp_l = grid.center(yi + HALF_H);
         const FaceRec *rec_b = a.rec + (size_t)b * a.nf;
         // pixel centres of the block's corner pixels, for the conservative edge cull
-        const float xa = pow2 ? __fmul_rn((float)(2 * wx0 + 1 - R), invR) : pix_center(wx0, R);
-        const float xb = pow2 ? __fmul_rn((float)(2 * wx1 + 1 - R), invR) : pix_center(wx1, R);
-        const float ya = pow2 ? __fmul_rn((float)(2 * wy0 + 1 - R), invR) : pix_center(wy0, R);
-        const float yb = pow2 ? __fmul_rn((float)(2 * wy1 + 1 - R), invR) : pix_center(wy1, R);
+        const float xa = grid.center(wx0), xb = grid.center(wx1);
+        const float ya = grid.center(wy0), yb = grid.center(wy1);
 
-        float depth_min = a.far_plane;
-        bool dexact = true;       // depth_min is the reference's value (not the cheap depth of the current winner)
-        int best = -1;
-        float bw0 = 0.f, bw1 = 0.f, bw2 = 0.f, bz0 = 0.f, bz1 = 0.f, bz2 = 0.f;
+        ZPix z_u = {a.far_plane, true, -1}, z_l = z_u;       // upper and lower pixel
 
         // software pipeline over the list: while group g is culled and evaluated, the records of
         // group g+1 and the ids of group g+2 are already in flight
         auto load_id = [&](int i) -> int { return i < n ? (overflow ? i : __ldg(list + i)) : -1; };
         int fid_next = load_id(lane);
         int fid_next2 = load_id(32 + lane);
-#if NR_CPASYNC_STAGE
-        int stage = 0;
-        auto stage_record = [&](int st, int f_) {
-            if (f_ >= 0) {
-                const float4 *rp = reinterpret_cast<const float4 *>(rec_b + f_);
-                const unsigned dst = (unsigned)__cvta_generic_to_shared(&s_stage[wid][st][lane][0]);
-                asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(rp));
-                asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst + 16), "l"(rp + 1));
-                asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst + 32), "l"(rp + 2));
-            }
-            asm volatile("cp.async.commit_group;" ::: "memory");
-        };
-        stage_record(0, fid_next);
-#else
         float4 n0 = make_float4(0.f, 0.f, 0.f, 0.f), n1 = n0, n2 = n0;
         if (fid_next >= 0) {
             const float4 *rp = reinterpret_cast<const float4 *>(rec_b + fid_next);
             n0 = __ldg(rp); n1 = __ldg(rp + 1); n2 = __ldg(rp + 2);
         }
-#endif
         for (int g = 0; g < n; g += 32) {
             // ---- one face per lane: cull against this warp's block, compact the survivors
             const int fid = fid_next;
-#if NR_CPASYNC_STAGE
-            fid_next = fid_next2;
-            stage_record(stage ^ 1, fid_next);                    // next group's records in flight ...
-            asm volatile("cp.async.wait_group 1;" ::: "memory");   // ... while this group's have landed
-            float4 q0 = make_float4(0.f, 0.f, 0.f, 0.f), q1 = q0, q2 = q0;
-            if (fid >= 0) {
-                q0 = s_stage[wid][stage][lane][0]; q1 = s_stage[wid][stage][lane][1]; q2 = s_stage[wid][stage][lane][2];
-            }
-            stage ^= 1;
-#else
             const float4 q0 = n0, q1 = n1, q2 = n2;
             fid_next = fid_next2;
             if (fid_next >= 0) {
                 const float4 *rp = reinterpret_cast<const float4 *>(rec_b + fid_next);
                 n0 = __ldg(rp); n1 = __ldg(rp + 1); n2 = __ldg(rp + 2);
             }
-#endif
             fid_next2 = load_id(g + 64 + lane);
             bool hit = false;
             if (fid >= 0) {
@@ -248,90 +243,103 @@ k_raster(const RasterArgs a) {
                 my_rec[slot][4] = make_float4(fast_rcp(z0), fast_rcp(z1), fast_rcp(z2),
                                               zreg ? fminf(z0, fminf(z1, z2)) : __int_as_float(0x7fc00000));
 #endif
-                // the face's pixel box (:94-97, exact by construction) as a bit mask over this block's 32
-                // pixels (bit = lane): the columns / rows it covers, relative to the block origin
+                // the face's pixel box (:94-97, exact by construction) as a bit mask over this block's 64
+                // pixels (bit = lane in .x for the upper half, in .y for the lower one): the columns / rows it
+                // covers, relative to the block origin.  A half's word is zero iff the box misses that half.
                 const uint32_t bx = __float_as_uint(q2.y), by = __float_as_uint(q2.z);
-                const int c0 = max((int)(bx & 0xffff) - wx0, 0), c1 = min((int)(bx >> 16) - wx0, WARP_BW - 1);
-                const int r0 = max((int)(by & 0xffff) - wy0, 0), r1 = min((int)(by >> 16) - wy0, WARP_BH - 1);
+                const int c0 = max((int)(bx & 0xffff) - wx0, 0), c1 = min((int)(bx >> 16) - wx0, BLK - 1);
+                const int r0 = max((int)(by & 0xffff) - wy0, 0), r1 = min((int)(by >> 16) - wy0, bh - 1);
                 const uint32_t cols = ((2u << c1) - 1u) & ~((1u << c0) - 1u);          // 8 bits
-                const uint32_t rows = ((2u << r1) - 1u) & ~((1u << r0) - 1u);          // 4 bits
-                my_bb[slot] = cols * ((rows * 0x00204081u) & 0x01010101u);              // row r -> bits 8r .. 8r+7
+                const uint32_t rows = ((2u << r1) - 1u) & ~((1u << r0) - 1u);          // 8 bits, 4 per half
+                // row r of a half -> bits 8r .. 8r+7
+                my_bb[slot] = make_uint2(cols * (((rows & 15u) * 0x00204081u) & 0x01010101u),
+                                         cols * (((rows >> 4) * 0x00204081u) & 0x01010101u));
             }
             __syncwarp();
             const int nh = __popc(m);
-            // ---- phase 1: coverage of every surviving face, one bit per face (cheap, all lanes)
-            unsigned inside = 0u;
-            // (branch-free: at least one lane of the block is inside every surviving face's pixel box, so the
-            // warp executes the edge functions anyway)
+            // ---- phase 1: coverage of every surviving face, one bit per face and pixel.  Every survivor's box
+            // touches at least one half; the record is read once for both.
+            unsigned in_u = 0u, in_l = 0u;
             for (int j = 0; j < nh; ++j) {
-                const bool in_box = (my_bb[j] >> lane) & 1u;
+                const uint2 bb = my_bb[j];       // the same words in every lane: the branches below do not diverge
                 const float4 A = my_rec[j][0], Bq = my_rec[j][1], Cq = my_rec[j][2];
-                // :107-116
-                const float c1 = __fmaf_rn(__fsub_rn(yp, A.y), Bq.z, -__fmul_rn(Bq.w, __fsub_rn(xp, A.x)));
-                const float c2 = __fmaf_rn(__fsub_rn(yp, A.w), Cq.x, -__fmul_rn(Cq.y, __fsub_rn(xp, A.z)));
-                const float c3 = __fmaf_rn(__fsub_rn(yp, Bq.y), Cq.z, -__fmul_rn(Cq.w, __fsub_rn(xp, Bq.x)));
-                const bool rejected = (__fmul_rn(c1, c2) < 0.f) | (__fmul_rn(c2, c3) < 0.f);
-                if (in_box && !rejected) inside |= 1u << j;
+                if (bb.x != 0u && (((bb.x >> lane) & 1u) != 0u) & edge_inside(xp, yp_u, A, Bq, Cq)) in_u |= 1u << j;
+                if (bb.y != 0u && (((bb.y >> lane) & 1u) != 0u) & edge_inside(xp, yp_l, A, Bq, Cq)) in_l |= 1u << j;
             }
             // ---- phase 2: every lane walks ITS OWN covering faces in list order (the z-test is
             // sequential per pixel only), so lanes evaluate different faces at the same time and the
-            // loop runs max-depth-complexity times instead of once per surviving face
-            while (inside) {
-                const int j = __ffs(inside) - 1;
-                inside &= inside - 1;
-                const float4 D = my_rec[j][3];
+            // loop runs max-depth-complexity times instead of once per surviving face; a lane walks its
+            // upper pixel's faces, then its lower pixel's
+#pragma unroll 1
+            for (int h = 0; h < 2; ++h) {
+                unsigned in = h ? in_l : in_u;
+                const float ypp = h ? yp_l : yp_u;
+                ZPix z = h ? z_l : z_u;
+                while (in) {
+                    const int j = __ffs(in) - 1;
+                    in &= in - 1;
+                    const float4 D = my_rec[j][3];
 #if NR_LAZY_Z
-                const float4 E = my_rec[j][4];
-                // surely depth_min < every corner depth (:124-126 skips the face); false for an irregular face
-                if (depth_min * (1.f + FAST_Z_REL) < E.w) continue;
-                const float4 A = my_rec[j][0], Bq = my_rec[j][1];
-                float w0, w1, w2;
-                raw_weights(xp, yp, A.x, A.y, A.z, A.w, Bq.x, Bq.y, w0, w1, w2);
-                if (E.w == E.w && weights_one_sign(w0, w1, w2)) {
-                    const float zf = fast_zp(w0, w1, w2, E.x, E.y, E.z);
-                    const float m = 2.f * FAST_Z_REL * fmaxf(zf, depth_min);     // error of zf plus that of depth_min
-                    const float t = depth_min - a.delta;
-                    // (every comparison is false for a NaN: such a candidate takes the exact path)
-                    if (zf < a.near_plane - m || zf > a.far_plane + m || zf > t + m) continue;      // :140-148 reject it
-                    if (zf > a.near_plane + m && zf < a.far_plane - m && zf < t - m) {              // ... accept it
-                        depth_min = zf;
-                        dexact = false;
-                        best = __float_as_int(D.w);
-                        bw0 = w0; bw1 = w1; bw2 = w2;
-                        bz0 = D.x; bz1 = D.y; bz2 = D.z;
-                        continue;
+                    const float4 E = my_rec[j][4];
+                    // surely depth_min < every corner depth (:124-126 skips the face); false for an irregular face
+                    if (z.depth_min * (1.f + FAST_Z_REL) < E.w) continue;
+                    const float4 A = my_rec[j][0], Bq = my_rec[j][1];
+                    float w0, w1, w2;
+                    raw_weights(xp, ypp, A.x, A.y, A.z, A.w, Bq.x, Bq.y, w0, w1, w2);
+                    if (E.w == E.w && weights_one_sign(w0, w1, w2)) {
+                        const float zf = fast_zp(w0, w1, w2, E.x, E.y, E.z);
+                        const float mg = 2.f * FAST_Z_REL * fmaxf(zf, z.depth_min);   // error of zf plus that of depth_min
+                        const float t = z.depth_min - a.delta;
+                        // (every comparison is false for a NaN: such a candidate takes the exact path)
+                        if (zf < a.near_plane - mg || zf > a.far_plane + mg || zf > t + mg) continue;   // :140-148 reject it
+                        if (zf > a.near_plane + mg && zf < a.far_plane - mg && zf < t - mg) {           // ... accept it
+                            z.depth_min = zf;
+                            z.dexact = false;
+                            z.best = __float_as_int(D.w);
+                            continue;
+                        }
+                    }
+                    // not clear: the reference's own arithmetic, against the exact running minimum (the
+                    // winner's record is read again: this only runs for near-ties)
+                    if (!z.dexact) {
+                        float v0, v1, v2, u0, u1, u2;
+                        winner_weights(rec_b, z.best, xp, ypp, v0, v1, v2, u0, u1, u2);
+                        z.depth_min = exact_zp_call(v0, v1, v2, u0, u1, u2);
+                        z.dexact = true;
+                    }
+                    if (z.depth_min < D.x && z.depth_min < D.y && z.depth_min < D.z) continue;    // :124-126
+                    const float zp = exact_zp_call(w0, w1, w2, D.x, D.y, D.z);                      // :129-139
+#else
+                    // :124-126
+                    if (z.depth_min < D.x && z.depth_min < D.y && z.depth_min < D.z) continue;
+                    const float4 A = my_rec[j][0], Bq = my_rec[j][1];
+                    // :129-136
+                    float w0, w1, w2;
+                    raw_weights(xp, ypp, A.x, A.y, A.z, A.w, Bq.x, Bq.y, w0, w1, w2);
+                    const float zp = exact_zp(w0, w1, w2, D.x, D.y, D.z);
+#endif
+                    // :139-142
+                    if (zp <= a.near_plane || a.far_plane <= zp) continue;
+                    // :145-148
+                    if (zp <= __fsub_rn(z.depth_min, a.delta)) {
+                        z.depth_min = zp;
+                        z.best = __float_as_int(D.w);
                     }
                 }
-                // not clear: the reference's own arithmetic, against the exact running minimum
-                if (!dexact) {
-                    depth_min = exact_zp_call(bw0, bw1, bw2, bz0, bz1, bz2);
-                    dexact = true;
-                }
-                if (depth_min < D.x && depth_min < D.y && depth_min < D.z) continue;      // :124-126
-                const float zp = exact_zp_call(w0, w1, w2, D.x, D.y, D.z);                 // :129-139
-#else
-                // :124-126
-                if (depth_min < D.x && depth_min < D.y && depth_min < D.z) continue;
-                const float4 A = my_rec[j][0], Bq = my_rec[j][1];
-                // :129-136
-                float w0, w1, w2;
-                raw_weights(xp, yp, A.x, A.y, A.z, A.w, Bq.x, Bq.y, w0, w1, w2);
-                const float zp = exact_zp(w0, w1, w2, D.x, D.y, D.z);
-#endif
-                // :139-142
-                if (zp <= a.near_plane || a.far_plane <= zp) continue;
-                // :145-148
-                if (zp <= __fsub_rn(depth_min, a.delta)) {
-                    depth_min = zp;
-                    best = __float_as_int(D.w);
-                    bw0 = w0; bw1 = w1; bw2 = w2;
-                    bz0 = D.x; bz1 = D.y; bz2 = D.z;
-                }
+                if (h) z_l = z;
+                else z_u = z;
             }
             __syncwarp();
         }
-        // ---------------------------------------------- epilogue: every pixel of the block is written
-        shade_block<RGB, AA, FULL>(a, b, xi, yi, valid, best, bw0, bw1, bw2, bz0, bz1, bz2, has_bg);
+        // ---------------------------------------------- epilogue: every pixel of the block is written, one
+        // 8x4 half at a time (shade_block's lane layout, its anti-aliasing quads lie within a half)
+#pragma unroll 1
+        for (int h = 0; h < (tall ? 2 : 1); ++h) {
+            const int yh = yi + h * HALF_H, best = h ? z_l.best : z_u.best;
+            float bw0 = 0.f, bw1 = 0.f, bw2 = 0.f, bz0 = 0.f, bz1 = 0.f, bz2 = 0.f;
+            if (best >= 0) winner_weights(rec_b, best, xp, h ? yp_l : yp_u, bw0, bw1, bw2, bz0, bz1, bz2);
+            shade_block<RGB, AA, FULL>(a, b, xi, yh, (xi < R) && (yh < R), best, bw0, bw1, bw2, bz0, bz1, bz2, has_bg);
+        }
     }   // items of this claim
     }   // claims
 }

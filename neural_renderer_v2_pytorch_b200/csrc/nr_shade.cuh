@@ -1,4 +1,4 @@
-// nr_shade.cuh -- device code shared by the two raster kernels (nr_raster.cu: one warp per 8x4 pixel block
+// nr_shade.cuh -- device code shared by the two raster kernels (nr_raster.cu: one warp per 8x8 pixel block
 // walking sorted tile lists; nr_raster_dense.cu: one CTA per tile, one thread per face, for meshes of small
 // triangles): the reference's depth arithmetic, the output fills and the fused shading epilogue.
 #pragma once
@@ -218,7 +218,7 @@ __device__ __forceinline__ void do_fill_item(const RasterArgs &a, const FillPlan
     }
 }
 
-// ---- epilogue: every pixel of a warp's 8x4 block is written ------------------------------------------------
+// ---- epilogue: every pixel of an 8x4 block is written ------------------------------------------------------
 // Called by ALL 32 lanes of a warp whose lane l owns pixel (xi, yi) = block origin + (l & 7, l >> 3) (the
 // anti-aliasing mean goes through quad shuffles).  best = winning face or -1, (bw0..2) its raw weight
 // numerators at this pixel, (bz0..2) its corner depths.  Fuses rasterize_cuda_kernel.cu:246-308 (weight map),

@@ -284,12 +284,18 @@ def _fim_cuda(nr, faces_np, R, near=0.1, far=100.0, backside=True):
     return fim.reshape(B, R, R).cpu().numpy(), wm.reshape(B, R, R, 3).cpu().numpy()
 
 
-def _check_vs_oracle(nr, faces_np, R, **kw):
-    fim, wm = _fim_cuda(nr, faces_np, R, **kw)
+def _check_vs_oracle(nr, faces_np, R, copies=1, **kw):
+    """The CUDA maps of faces_np [B, nf, 3, 3] against the C oracle's.  The GPU renders the B views `copies`
+    times over in one call (an int, or a function of the oracle's face_index_map: see
+    test_gpu_raster_blocks.py); the oracle runs once and every copy is compared with it."""
     want = oracle.face_index_map(faces_np, R, kw.get("near", 0.1), kw.get("far", 100.0), kw.get("backside", True))
+    want_wm = oracle.weight_map(faces_np, want)
+    k = copies(want) if callable(copies) else copies
+    if k != 1:
+        faces_np, want, want_wm = (np.concatenate([a] * k) for a in (faces_np, want, want_wm))
+    fim, wm = _fim_cuda(nr, faces_np, R, **kw)
     nbad = int((fim != want).sum())
     assert nbad == 0, "face_index_map: %d / %d pixels differ" % (nbad, fim.size)
-    want_wm = oracle.weight_map(faces_np, want)
     assert np.array_equal(wm, want_wm), "weight_map differs"
     # the fused forward itself, with both binning paths (one kernel per view / general multi-kernel)
     from neural_renderer_v2_pytorch_b200 import rasterize as rz
@@ -809,29 +815,39 @@ def test_reference_backward_case1_with_its_own_target(nr):
     raise AssertionError("IoU loss %.4f after 350 iterations" % float(iou.detach()))
 
 
-@pytest.mark.parametrize("S,aa,fine,general", [(64, False, False, False), (36, True, False, False), (40, True, True, True),
-                                                (50, False, True, True), (64, True, False, True), (50, False, "dense", True),
-                                                (36, True, "dense", True)])
-def test_kernels_stay_inside_their_buffers(nr, S, aa, fine, general):
+@pytest.mark.parametrize("S,aa,fine,general,height", [
+    pytest.param(*c[:4], c[4] if len(c) > 4 else "8x4", id="-".join(str(x) for x in c)) for c in [
+        (64, False, False, False), (36, True, False, False), (40, True, True, True), (50, False, True, True),
+        (64, True, False, True), (50, False, "dense", True), (36, True, "dense", True),
+        (64, False, False, False, "8x8"), (64, False, True, True, "8x8"), (36, True, False, False, "8x8"),
+        (50, False, False, False, "8x8"), (64, False, False, False, "8x8-no-pair-room")]])
+def test_kernels_stay_inside_their_buffers(nr, S, aa, fine, general, height):
     """No sanitizer on this pool: every output of the forward / backward is carved out of a larger
     poisoned allocation and the guard words on both sides must survive (vector and scalar fill paths,
-    16x16 and 8x8 tiles, one-kernel and general binning, zero-fill chunks, gradient atomics)."""
+    16x16 and 8x8 tiles, one-kernel and general binning, zero-fill chunks, gradient atomics).  The tile
+    rasterizer runs 8x4 or 8x8 warp blocks (`height`: three views, or as many copies of them as
+    test_gpu_raster_blocks.copies asks for), with or without room for the (tile, face) pairs."""
     import ctypes
     from neural_renderer_v2_pytorch_b200 import _lib, rasterize as rz
+    from test_gpu_raster_blocks import copies
     L = _lib.lib()
     d = np.load(os.path.join(GOLDEN, "teapot.npz"))
     B, G_ = 3, 4096
     g = torch.Generator().manual_seed(S)
     vw = torch.from_numpy(d["vertices"])[None].repeat(B, 1, 1)
     eye = nr.get_points_from_angles(torch.full((B,), 2.732), torch.rand(B, generator=g) * 80 - 20, torch.rand(B, generator=g) * 360)
-    v = nr.perspective(nr.look_at(vw, eye)).cuda().contiguous()
-    faces = torch.from_numpy(d["faces"]).cuda()
+    v = nr.perspective(nr.look_at(vw, eye)).contiguous()
+    faces = torch.from_numpy(d["faces"])
     vt_np, ft_np, tex_np = nr.create_textures(faces.shape[0], 2)
-    tex = torch.rand((B,) + tex_np.shape, generator=g).cuda()
-    vt = torch.from_numpy(vt_np)[None].repeat(B, 1, 1).cuda()
-    ft = torch.from_numpy(ft_np).cuda()
+    tex = torch.rand((B,) + tex_np.shape, generator=g)
     R = 2 * S if aa else S
     dense, fine = fine == "dense", fine is True
+    if not dense:
+        k = copies(oracle.face_index_map(v[:, faces.long()].numpy(), R), height[:3], fine)
+        B, v, tex = B * k, torch.cat([v] * k), torch.cat([tex] * k)
+    v, faces, tex = v.cuda().contiguous(), faces.cuda(), tex.cuda()
+    vt = torch.from_numpy(vt_np)[None].repeat(B, 1, 1).cuda()
+    ft = torch.from_numpy(ft_np).cuda()
     flags = (_lib.NR_DRAW_RGB | _lib.NR_DRAW_SILHOUETTES | _lib.NR_DRAW_BACKSIDE | (_lib.NR_ANTI_ALIASING if aa else 0) |
              (_lib.NR_FINE_TILES if fine else 0) | (_lib.NR_GENERAL_BINNING if general else 0) |
              (_lib.NR_DENSE_RASTER if dense else 0))
@@ -840,7 +856,7 @@ def test_kernels_stay_inside_their_buffers(nr, S, aa, fine, general):
                             tex_height=tex.shape[2], tex_width=tex.shape[3])
     tile = 8 if fine else 16
     ntx = (R + tile - 1) // tile
-    cap = 8 * B * faces.shape[0]
+    cap = 0 if height.endswith("no-pair-room") else 8 * B * faces.shape[0]
     POISON_I, POISON_F = 0x5a5a5a5a, 12345.5
 
     def guarded(n, dtype):

@@ -75,6 +75,10 @@ enum {
                                  above 4096 pixels (more than a few per cent of the faces: drop the flag),
                                  overflow = 1 when the candidate pool (pair_capacity / 4 entries) was too small
                                  (still exact, slower). */
+#define NR_VIEW_FACES 1024    /* forward and backward: one mesh topology per view.  `faces` is [B, nf, 3] and, with
+                                 NR_DRAW_RGB, `faces_textures` is [B, nf, 3] as well; view b reads row b of both.
+                                 Views with fewer faces pad their rows with a degenerate face (three equal indices,
+                                 e.g. 0 0 0): it is never drawn and gets no gradient.  faces must not be NULL. */
 
 /* Mirrors RasterizeHyperparam (rasterize_param.py:13-33) plus the tensor extents. */
 typedef struct nrRasterConfig {
@@ -184,9 +188,10 @@ NR_API size_t nr_workspace_bytes(const nrRasterConfig *cfg, int64_t pair_capacit
  *
  *   vertices            [B, nv, 3]   screen-space x, y in [-1, 1], z = depth
  *   faces               [nf, 3]      vertex ids; NULL means face f uses vertices 3f, 3f+1, 3f+2
- *                                    (i.e. `vertices` is the gathered [B, nf, 3, 3] tensor)
+ *                                    (i.e. `vertices` is the gathered [B, nf, 3, 3] tensor);
+ *                                    [B, nf, 3] with NR_VIEW_FACES
  *   vertices_textures   [B, nvt, 2]  texel coordinates           (NR_DRAW_RGB only)
- *   faces_textures      [nf, 3]      ids into vertices_textures  (NR_DRAW_RGB only)
+ *   faces_textures      [nf, 3]      ids into vertices_textures  (NR_DRAW_RGB only; [B, nf, 3] with NR_VIEW_FACES)
  *   textures            [B, 3, H, W]                             (NR_DRAW_RGB only)
  *   face_index_map      [B, R, R]    out, -1 on background (never NULL)
  *   weight_map          [B, R, R, 3] out, optional (NULL to skip)

@@ -27,6 +27,7 @@ NR_GENERAL_BINNING = 64
 NR_SPARSE_MAPS = 128
 NR_FINE_TILES = 256
 NR_DENSE_RASTER = 512
+NR_VIEW_FACES = 1024
 
 # every symbol include/nr_b200.h declares (tests/test_abi.py checks header <-> library <-> this list)
 SYMBOLS = (

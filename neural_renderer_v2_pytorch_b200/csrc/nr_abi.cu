@@ -121,11 +121,18 @@ int tile_edge(const nrRasterConfig *cfg) {
     return ((cfg->flags & NR_FINE_TILES) && !(cfg->flags & NR_DENSE_RASTER)) ? nr::FINE_TILE : nr::TILE;
 }
 
+// ints from one view's face rows to the next: every view reads the same [nf, 3] rows, or its own of [B, nf, 3]
+int view_face_stride(const nrRasterConfig *cfg) {
+    return (cfg->flags & NR_VIEW_FACES) ? 3 * cfg->num_faces : 0;
+}
+
 int check_config(const nrRasterConfig *cfg) {
     if (!cfg) return fail(NR_ERR_INVALID_ARGUMENT, "config is NULL");
     if (cfg->batch < 0 || cfg->num_vertices < 0 || cfg->num_faces < 0 || cfg->image_size <= 0)
         return fail(NR_ERR_INVALID_ARGUMENT, "negative extent or image_size <= 0");
     if (cfg->batch > 65535) return fail(NR_ERR_INVALID_ARGUMENT, "batch > 65535");
+    if ((cfg->flags & NR_VIEW_FACES) && cfg->num_faces > 0x7fffffff / 3)
+        return fail(NR_ERR_INVALID_ARGUMENT, "NR_VIEW_FACES: a view's face rows exceed 2^31 ints");
     const long long R = (long long)cfg->image_size * ((cfg->flags & NR_ANTI_ALIASING) ? 2 : 1);
     if (R > 32768) return fail(NR_ERR_INVALID_ARGUMENT, "internal resolution > 32768");
     if (!(cfg->flags & (NR_DRAW_RGB | NR_DRAW_SILHOUETTES | NR_DRAW_DEPTH)))
@@ -222,6 +229,7 @@ int nr_rasterize_forward(const nrRasterConfig *cfg, const float *vertices, const
     const int R = cfg->image_size * (aa ? 2 : 1);
     if (!vertices && cfg->batch * cfg->num_faces > 0) return fail(NR_ERR_INVALID_ARGUMENT, "vertices is NULL");
     if (!face_index_map) return fail(NR_ERR_INVALID_ARGUMENT, "face_index_map is NULL");
+    if ((cfg->flags & NR_VIEW_FACES) && !faces) return fail(NR_ERR_INVALID_ARGUMENT, "NR_VIEW_FACES needs faces [B, nf, 3]");
     if (rgb && (!vertices_textures || !faces_textures || !textures))
         return fail(NR_ERR_INVALID_ARGUMENT, "NR_DRAW_RGB needs vertices_textures, faces_textures and textures");
     if (rgb && (cfg->tex_height <= 0 || cfg->tex_width <= 0 || cfg->num_tex_vertices <= 0))
@@ -251,6 +259,7 @@ int nr_rasterize_forward(const nrRasterConfig *cfg, const float *vertices, const
     nr::BinningArgs ba;
     ba.verts = vertices;
     ba.faces = faces;
+    ba.face_stride = view_face_stride(cfg);
     ba.B = cfg->batch;
     ba.nv = cfg->num_vertices;
     ba.nf = cfg->num_faces;
@@ -302,6 +311,7 @@ int nr_rasterize_forward(const nrRasterConfig *cfg, const float *vertices, const
     if ((uintptr_t)aux_map & 7) return fail(NR_ERR_INVALID_ARGUMENT, "aux_map not 8-byte aligned");
     ra.aux = aux_map;
     ra.faces = faces;
+    ra.face_stride = ba.face_stride;
     ra.nv = cfg->num_vertices;
     ra.verts = vertices;
     ra.zbuf = c.zbuf;
@@ -383,12 +393,14 @@ int nr_rasterize_backward_lights(const nrRasterConfig *cfg, const float *vertice
     const bool aa = cfg->flags & NR_ANTI_ALIASING, rgb = cfg->flags & NR_DRAW_RGB;
     if (!vertices || !face_index_map || !images_internal || !grad_images || !grad_vertices)
         return fail(NR_ERR_INVALID_ARGUMENT, "backward: a required pointer is NULL");
+    if ((cfg->flags & NR_VIEW_FACES) && !faces) return fail(NR_ERR_INVALID_ARGUMENT, "NR_VIEW_FACES needs faces [B, nf, 3]");
     if (rgb && (!vertices_textures || !faces_textures || !textures))
         return fail(NR_ERR_INVALID_ARGUMENT, "NR_DRAW_RGB needs vertices_textures, faces_textures and textures");
     if (cfg->batch == 0) return NR_OK;
     nr::BackwardArgs a;
     a.verts = vertices;
     a.faces = faces;
+    a.face_stride = view_face_stride(cfg);
     a.vt = vertices_textures;
     a.ft = faces_textures;
     a.tex = textures;

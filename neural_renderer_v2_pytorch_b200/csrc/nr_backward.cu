@@ -467,10 +467,12 @@ k_backward(const __grid_constant__ BackwardArgs a) {
     constexpr bool LIT = (CT == 0);      // lights only in the generic variants (keeps the common ones small)
     const bool has_z = rgb || (a.flags & FLAG_DEPTH) != 0;
     if (fg) {
+        // this view's face rows: its own with NR_VIEW_FACES (face_stride = 3 nf), else the shared ones
+        const size_t frow = (size_t)b * a.face_stride + 3 * (size_t)f;
         if (a.faces) {
-            vid[0] = __ldg(a.faces + 3 * (size_t)f);
-            vid[1] = __ldg(a.faces + 3 * (size_t)f + 1);
-            vid[2] = __ldg(a.faces + 3 * (size_t)f + 2);
+            vid[0] = __ldg(a.faces + frow);
+            vid[1] = __ldg(a.faces + frow + 1);
+            vid[2] = __ldg(a.faces + frow + 2);
         } else {
             vid[0] = 3 * f; vid[1] = 3 * f + 1; vid[2] = 3 * f + 2;
         }
@@ -507,7 +509,7 @@ k_backward(const __grid_constant__ BackwardArgs a) {
         if (rgb) {
             const float g_lit[3] = {gcen[0], gcen[1], gcen[2]};
             if (g_lit[0] != 0.f || g_lit[1] != 0.f || g_lit[2] != 0.f) {
-                const int32_t *fti = a.ft + 3 * (size_t)f;
+                const int32_t *fti = a.ft + frow;
                 const float *vtb = a.vt + (size_t)b * a.nvt * 2;
                 int tvid[3];
                 float u[3], v[3];

@@ -21,7 +21,7 @@
 namespace nr {
 
 __global__ void __launch_bounds__(256)
-k_setup_count(const float *__restrict__ verts, const int32_t *__restrict__ faces, int B, int nv,
+k_setup_count(const float *__restrict__ verts, const int32_t *__restrict__ faces, int face_stride, int B, int nv,
               int nf, int R, int draw_backside, FaceRec *__restrict__ rec,
               int *__restrict__ tile_count, int ntx, int tsh, BinHeader *__restrict__ hdr) {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -29,7 +29,8 @@ k_setup_count(const float *__restrict__ verts, const int32_t *__restrict__ faces
     const int b = (int)(idx / nf), f = (int)(idx % nf);
     FaceRec r;
     int xlo, xhi, ylo, yhi;
-    const bool alive = make_face_record(verts + (size_t)b * nv * 3, faces, f, nv, R, draw_backside, r, xlo, xhi, ylo, yhi, hdr);
+    const bool alive = make_face_record(verts + (size_t)b * nv * 3, faces + (size_t)b * face_stride, f, nv, R, draw_backside, r,
+                                        xlo, xhi, ylo, yhi, hdr);
     rec[idx] = r;
     if (!alive) return;
 
@@ -196,7 +197,7 @@ __device__ __forceinline__ void warp_rank_sort(const int *src, int n, int32_t *d
 }
 
 __global__ void __launch_bounds__(BINVIEW_THREADS, 1)
-k_bin_view(const float *__restrict__ verts, const int32_t *__restrict__ faces, int nv, int nf, int R,
+k_bin_view(const float *__restrict__ verts, const int32_t *__restrict__ faces, int face_stride, int nv, int nf, int R,
            int draw_backside, int ntx, FaceRec *__restrict__ rec, int *__restrict__ tile_count,
            int32_t *__restrict__ pairs, long long pair_capacity, BinHeader *__restrict__ hdr,
            int32_t *__restrict__ tile_list) {
@@ -231,7 +232,8 @@ k_bin_view(const float *__restrict__ verts, const int32_t *__restrict__ faces, i
     for (int f = f_begin + tid; f < f_end; f += BINVIEW_THREADS) {
         FaceRec r;
         int xlo, xhi, ylo, yhi;
-        const bool alive = make_face_record(vb, faces, f, nv, R, draw_backside, r, xlo, xhi, ylo, yhi, hdr);
+        // (an int offset: b * 3 nf < 65536 * 3 * BINVIEW_MAX_FACES < 2^31, and no 64-bit pointer held across the kernel)
+        const bool alive = make_face_record(vb, faces + b * face_stride, f, nv, R, draw_backside, r, xlo, xhi, ylo, yhi, hdr);
         rec_b[f] = r;
         if (!alive) continue;
         const int tx0 = xlo / TILE, tx1 = xhi / TILE, ty0 = ylo / TILE, ty1 = yhi / TILE;
@@ -623,7 +625,7 @@ cudaError_t launch_binning(const BinningArgs &a, cudaStream_t stream) {
         cfg.numAttrs = 1;
         {
             ProfScope p(PROF_SETUP, stream);
-            e = cudaLaunchKernelEx(&cfg, k_bin_view, a.verts, a.faces, a.nv, a.nf, a.R, a.draw_backside, a.ntx, a.rec,
+            e = cudaLaunchKernelEx(&cfg, k_bin_view, a.verts, a.faces, a.face_stride, a.nv, a.nf, a.R, a.draw_backside, a.ntx, a.rec,
                                    a.tile_count, a.pairs, a.pair_capacity, a.hdr, a.tile_list);
         }
         if (e == cudaSuccess) return e;
@@ -642,7 +644,7 @@ cudaError_t launch_binning(const BinningArgs &a, cudaStream_t stream) {
     if (nface > 0) {
         const unsigned blocks = (unsigned)((nface + 255) / 256);
         ProfScope p(PROF_SETUP, stream);
-        k_setup_count<<<blocks, 256, 0, stream>>>(a.verts, a.faces, a.B, a.nv, a.nf, a.R,
+        k_setup_count<<<blocks, 256, 0, stream>>>(a.verts, a.faces, a.face_stride, a.B, a.nv, a.nf, a.R,
                                                   a.draw_backside, a.rec, a.tile_count, a.ntx, a.tile_shift, a.hdr);
     }
     {

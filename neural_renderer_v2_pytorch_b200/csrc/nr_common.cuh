@@ -136,7 +136,7 @@ __device__ __forceinline__ int last_pixel_le(float v, const PixGrid &g) {
     return i;
 }
 
-// Record of face f of one view (vb = that view's vertices) and its exact pixel box; returns false for
+// Record of face f of one view (vb = that view's vertices, faces = its face rows) and its exact pixel box; returns false for
 // a face no pixel can accept (its record then carries the dead box).
 __device__ __forceinline__ bool make_face_record(const float *__restrict__ vb, const int32_t *__restrict__ faces,
                                                  int f, int nv, int R, int draw_backside, FaceRec &r, int &xlo,

@@ -27,6 +27,7 @@ struct BinningArgs {
     const float *verts;
     const int32_t *faces;   // may be null: face f = vertices 3f..3f+2
     int B, nv, nf, R, draw_backside, ntx;
+    int face_stride;        // ints between the face rows of consecutive views: 3 nf (NR_VIEW_FACES) or 0
     FaceRec *rec;
     int *tile_count, *tile_offset, *tile_cursor;
     int32_t *pairs;
@@ -50,7 +51,7 @@ struct RasterArgs {
     int B, nf, R, S, ntx, C, flags;
     float near_plane, far_plane, eps, delta;
     const float *vt;        // [B, nvt, 2]
-    const int32_t *ft;      // [nf, 3]
+    const int32_t *ft;      // [nf, 3], or [B, nf, 3] with face_stride
     const float *tex;       // [B, 3, H, W]
     int nvt, H, W;
     int32_t *fim;           // [B, R, R]
@@ -59,8 +60,9 @@ struct RasterArgs {
     float *images;          // [B, C, S, S] or null (compat call renders no image)
     float *internal;        // [B, C, R, R] (AA) or null
     float *aux;             // [B, R, R, 6 (rgb) or 3] forward -> backward state at foreground pixels, or null
-    const int32_t *faces;   // [nf, 3] vertex ids (null: 3f..3f+2), only read when lights are on
+    const int32_t *faces;   // [nf, 3] vertex ids (null: 3f..3f+2), or [B, nf, 3] with face_stride
     int nv;
+    int face_stride;        // ints between the face (and texture-face) rows of consecutive views: 3 nf or 0
     LightArgs lights;
     int fine;               // 8x8 tiles (ntx and the tile list are in those units)
     int sparse_maps;        // fim / internal only where the backward reads them (see NR_SPARSE_MAPS)
@@ -85,7 +87,7 @@ cudaError_t launch_raster_zbuf(const RasterArgs &a, cudaStream_t stream);      /
 
 struct BackwardArgs {
     const float *verts;     // [B, nv, 3]
-    const int32_t *faces;   // [nf, 3] or null
+    const int32_t *faces;   // [nf, 3] or null, or [B, nf, 3] with face_stride
     const float *vt;
     const int32_t *ft;
     const float *tex;
@@ -102,6 +104,7 @@ struct BackwardArgs {
     float det_scale;
     LightArgs lights;
     int B, nv, nf, R, S, ntx, C, flags, nvt, H, W;
+    int face_stride;        // ints between the face (and texture-face) rows of consecutive views: 3 nf or 0
     float eps;
     // gradient of the light data [L, B, 8] (colour 0..2, direction 3..5, alpha 6), accumulated; null = none.
     // Read by the lit variants only.  det_light: its fixed-point accumulator in deterministic mode.

@@ -384,7 +384,10 @@ cudaError_t launch_raster(const RasterArgs &a, cudaStream_t stream) {
     const int grid = (int)(tiles < (long long)a.sm_count * 8 ? tiles : (long long)a.sm_count * 8);
     const bool rgb = (a.flags & FLAG_RGB) != 0, aa = (a.flags & FLAG_AA) != 0;
     // everything optional goes to the FULL variants
-    const bool full = a.lights.num > 0 || a.lights.backgrounds || a.wmap || a.dmap || !a.images || (a.R & 15);
+    // colour with per-view faces (NR_VIEW_FACES) also takes the full variants: only they add the view's row offset to
+    // faces_textures, which costs the plain colour variant (config 2) spill traffic
+    const bool full = a.lights.num > 0 || a.lights.backgrounds || a.wmap || a.dmap || !a.images || (a.R & 15) ||
+                      (rgb && a.face_stride != 0);
     ProfScope p(PROF_RASTER, stream);
     if (a.fine) {       // dense meshes: the full-featured kernels over 8x8 tiles
         switch ((rgb ? 1 : 0) | (aa ? 2 : 0)) {

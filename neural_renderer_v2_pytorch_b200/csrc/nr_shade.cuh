@@ -299,7 +299,8 @@ __device__ __forceinline__ void shade_block(const RasterArgs &a, int b, int xi, 
         if (RGB) {
             float rgb[3] = {0.f, 0.f, 0.f};
             if (fg) {
-                const int32_t *fti = a.ft + 3 * (size_t)best;
+                // (per-view faces_textures: the launchers send those calls to the FULL variants)
+                const int32_t *fti = a.ft + (FULL ? (size_t)b * a.face_stride : 0) + 3 * (size_t)best;
                 const float *vtb = a.vt + (size_t)b * a.nvt * 2;
                 float u[3], v[3];
                 // a texture-vertex index outside [0, nvt) (an IndexError in the reference, rasterize.py:246)
@@ -328,9 +329,10 @@ __device__ __forceinline__ void shade_block(const RasterArgs &a, int b, int xi, 
                     // smooth normal map (rasterize.py:186-187) and light accumulation (:252-283)
                     float n[3] = {0.f, 0.f, 0.f}, cw[3];
                     const float *vnb = a.lights.vnormals + (size_t)b * a.nv * 3;
+                    const int32_t *fr = a.faces ? a.faces + (size_t)b * a.face_stride + 3 * (size_t)best : nullptr;
 #pragma unroll
                     for (int k = 0; k < 3; ++k) {
-                        const int vid = a.faces ? __ldg(a.faces + 3 * (size_t)best + k) : 3 * best + k;
+                        const int vid = fr ? __ldg(fr + k) : 3 * best + k;
 #pragma unroll
                         for (int c2 = 0; c2 < 3; ++c2) n[c2] = __fadd_rn(n[c2], __fmul_rn(q[k], __ldg(vnb + 3 * (size_t)vid + c2)));
                     }

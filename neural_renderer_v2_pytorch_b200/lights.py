@@ -104,9 +104,31 @@ def vertex_normals(vertices, faces, deterministic=False):
 
     index_add sums with float atomics on CUDA, so the last bits vary from run to run.  ``deterministic`` sums
     with index_put(accumulate=True) instead, which sorts the indices and adds in a fixed order: the normals,
-    and through them the lit images and every lit gradient, are then bit-identical from run to run."""
+    and through them the lit images and every lit gradient, are then bit-identical from run to run.
+
+    ``faces`` may also be [B,nf,3], one topology per view: view b's normals then come from row b alone, equal to
+    a call with that view and row (the sums run over the flattened [B*nv] vertices, each view at its offset)."""
     import torch.nn.functional as F
     idx = faces.long()
+    if idx.ndim == 3:
+        B, nv = vertices.shape[:2]
+        fv = vertices[torch.arange(B, device=idx.device)[:, None, None], idx]       # [B,nf,3,3]
+        n = torch.linalg.cross(fv[:, :, 1] - fv[:, :, 0], fv[:, :, 2] - fv[:, :, 1], dim=-1)
+        once1 = (idx[:, :, 1] != idx[:, :, 0]).to(n.dtype)[..., None]
+        once2 = ((idx[:, :, 2] != idx[:, :, 0]) & (idx[:, :, 2] != idx[:, :, 1])).to(n.dtype)[..., None]
+        flat = idx + (torch.arange(B, device=idx.device) * nv)[:, None, None]   # ids into [B*nv]
+        vflat = vertices.reshape(B * nv, 3)
+        if deterministic:
+            # per view the same order of contributions as the [nf,3] call: corner 0 of every face, then 1, then 2
+            vals = torch.cat([n, n * once1, n * once2], dim=1).reshape(-1, 3)
+            ids = torch.cat([flat[:, :, 0], flat[:, :, 1], flat[:, :, 2]], dim=1).reshape(-1)
+            vn = torch.zeros_like(vflat).index_put((ids,), vals, accumulate=True)
+        else:
+            vn = torch.zeros_like(vflat)
+            vn = vn.index_add(0, flat[:, :, 0].reshape(-1), n.reshape(-1, 3))
+            vn = vn.index_add(0, flat[:, :, 1].reshape(-1), (n * once1).reshape(-1, 3))
+            vn = vn.index_add(0, flat[:, :, 2].reshape(-1), (n * once2).reshape(-1, 3))
+        return F.normalize(vn.reshape(B, nv, 3), dim=2)
     fv = vertices[:, idx]                                            # [B,nf,3,3]
     n = torch.linalg.cross(fv[:, :, 1] - fv[:, :, 0], fv[:, :, 2] - fv[:, :, 1], dim=-1)
     once1 = (idx[:, 1] != idx[:, 0]).to(n.dtype)[None, :, None]

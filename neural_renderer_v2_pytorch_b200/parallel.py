@@ -32,7 +32,7 @@ def shard_range(num_views, rank=None, world_size=None):
 
 
 def shard_views(tensor, rank=None, world_size=None):
-    """Slice dim 0 (views) of ``tensor`` for this rank."""
+    """Slice dim 0 (views) of ``tensor`` for this rank.  Per-view faces [B, nf, 3] are sharded like the vertices."""
     b, e = shard_range(tensor.shape[0], rank, world_size)
     return tensor[b:e]
 

@@ -416,11 +416,13 @@ class _Rasterize(torch.autograd.Function):
 
 
 def _prepare(vertices, faces, params, hyperparams):
-    # shape checks of rasterize.py:195-205 (AssertionError, like the reference)
+    # shape checks of rasterize.py:195-205 (AssertionError, like the reference).  Beyond the reference, faces (and
+    # faces_textures) may be [B, nf, 3]: one topology per view (NR_VIEW_FACES, DESIGN.md "API notes").
     assert vertices.ndim == 3
     assert vertices.shape[2] == 3
-    assert faces.ndim == 2
-    assert faces.shape[1] == 3
+    assert faces.ndim in (2, 3)
+    assert faces.shape[-1] == 3
+    assert faces.ndim == 2 or faces.shape[0] == vertices.shape[0]
     dev = vertices.device
     bg = None
     if hyperparams.draw_rgb:
@@ -442,27 +444,35 @@ def _prepare(vertices, faces, params, hyperparams):
     faces = torch.as_tensor(faces)
     faces_d = _i32c(faces).to(dev)
     B, nv = vertices.shape[:2]
-    nf = faces_d.shape[0]
+    nf = faces_d.shape[-2]
     _validate_indices(faces, nv, "faces")
+    view_faces = faces_d.ndim == 3
     vt = ft = tex = None
     nvt = H = W = 0
     if hyperparams.draw_rgb:
         assert params.vertices_textures.ndim == 3
         assert params.vertices_textures.shape[2] == 2
-        assert params.faces_textures.ndim == 2
-        assert params.faces_textures.shape[1] == 3
+        assert params.faces_textures.ndim in (2, 3)
+        assert params.faces_textures.shape[-1] == 3
         assert params.textures.ndim == 4
         assert params.textures.shape[1] == 3
         vt, tex = params.vertices_textures, params.textures
         _require_cuda(vt, "vertices_textures")
         _require_cuda(tex, "textures")
         assert vt.shape[0] == B and tex.shape[0] == B
-        assert params.faces_textures.shape[0] == nf
+        assert params.faces_textures.shape[-2] == nf
+        assert params.faces_textures.ndim == 2 or params.faces_textures.shape[0] == B
         ft = _i32c(torch.as_tensor(params.faces_textures)).to(dev)
         nvt, H, W = vt.shape[1], tex.shape[2], tex.shape[3]
         _validate_indices(torch.as_tensor(params.faces_textures), nvt, "faces_textures")
-    cfg = _make_config(B, nv, nf, int(hyperparams.image_size), _flags_of(hyperparams), hyperparams,
-                       nvt, H, W)
+        view_faces = view_faces or ft.ndim == 3
+        if view_faces:
+            ft = ft.expand(B, nf, 3).contiguous()
+    if view_faces:
+        # the kernels read row b of both index tensors for view b: the shared one is expanded (12 B nf bytes)
+        faces_d = faces_d.expand(B, nf, 3).contiguous()
+    cfg = _make_config(B, nv, nf, int(hyperparams.image_size),
+                       _flags_of(hyperparams) | (_lib.NR_VIEW_FACES if view_faces else 0), hyperparams, nvt, H, W)
     light_pack = vn = None
     if hyperparams.draw_rgb and params.lights is not None:      # an empty list renders black, rasterize.py:252-283
         # shading: per-vertex normals by differentiable torch ops (O(nv + nf)), the per-pixel part in the kernels
@@ -472,7 +482,7 @@ def _prepare(vertices, faces, params, hyperparams):
 
 
 def rasterize_core(vertices, faces, params: RasterizeParam, hyperparams: RasterizeHyperparam):
-    """``rasterize.py:194-329``. vertices [B,nv,3] screen space, faces [nf,3] -> images [B,C,S,S]."""
+    """``rasterize.py:194-329``. vertices [B,nv,3] screen space, faces [nf,3] or [B,nf,3] -> images [B,C,S,S]."""
     cfg, faces_d, vt, ft, tex, vn, light_pack, bg = _prepare(vertices, faces, params, hyperparams)
     light_types, light_data = light_pack if light_pack is not None else (None, None)
     return _Rasterize.apply(vertices, vt, tex, vn, bg, light_data, faces_d, ft, cfg, light_types)

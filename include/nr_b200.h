@@ -246,9 +246,14 @@ NR_API int nr_rasterize_forward(const nrRasterConfig *cfg, const float *vertices
  *   grad_vertices_textures [B, nvt, 2] out, accumulated, optional
  *   deterministic_scratch  only with NR_DETERMINISTIC in cfg->flags: nr_deterministic_scratch_bytes(cfg)
  *                       zero-filled bytes.  Contributions are then rounded once to 64-bit fixed point
- *                       (x 2^32) and summed with integer atomics, so the gradients are bit-identical from
- *                       run to run (float atomics depend on arrival order).  Valid while every |sum| < 2.1e9;
- *                       absolute resolution 2.3e-10.  Covers grad_vertex_normals (lights) as well.
+ *                       and summed with integer atomics, so the gradients are bit-identical from run to run
+ *                       (float atomics depend on arrival order).  The unit is chosen per view on the device:
+ *                       2^(E_b - 32), with m_b = max |grad_images| over view b's finite values in
+ *                       [2^(E_b - 1), 2^E_b) (E_b = 0 for an all-zero view).  So the resolution is
+ *                       <= 4.7e-10 m_b and the results are valid while every |sum| < 2^(31 + E_b) (>= 2.1e9 m_b);
+ *                       scaling G by a power of two scales the gradients exactly, and a view's bits do not
+ *                       depend on the other views of the call.  NaN and +-inf contributions are summed as floats
+ *                       and come out as with float atomics.  Covers grad_vertex_normals and grad_light_data.
  */
 NR_API int nr_rasterize_backward(const nrRasterConfig *cfg, const float *vertices, const int32_t *faces,
                           const float *vertices_textures, const int32_t *faces_textures,

@@ -199,14 +199,18 @@ int nr_event_synchronize(void *event) {
     return e == cudaSuccess ? NR_OK : fail_cuda(e, "cudaEventSynchronize");
 }
 
+// 64-bit accumulators of the deterministic scratch: vertices, textures, vertices_textures, vertex normals (lights),
+// back to back.  The B per-view maxima of |grad_images| (BackwardArgs::det_gmax) follow them.
+static size_t det_fixed_elems(const nrRasterConfig *cfg) {
+    return (size_t)cfg->batch * cfg->num_vertices * 3 +
+           (size_t)cfg->batch * 3 * cfg->tex_height * cfg->tex_width +
+           (size_t)cfg->batch * cfg->num_tex_vertices * 2 +
+           (size_t)cfg->batch * cfg->num_vertices * 3;
+}
+
 size_t nr_deterministic_scratch_bytes(const nrRasterConfig *cfg) {
     if (!cfg) return 0;
-    // vertices, textures, vertices_textures, vertex normals (lights), back to back
-    const size_t n = (size_t)cfg->batch * cfg->num_vertices * 3 +
-                     (size_t)cfg->batch * 3 * cfg->tex_height * cfg->tex_width +
-                     (size_t)cfg->batch * cfg->num_tex_vertices * 2 +
-                     (size_t)cfg->batch * cfg->num_vertices * 3;
-    return n * sizeof(long long);
+    return det_fixed_elems(cfg) * sizeof(long long) + (((size_t)cfg->batch * sizeof(unsigned) + 7) & ~(size_t)7);
 }
 
 size_t nr_workspace_bytes(const nrRasterConfig *cfg, int64_t pair_capacity) {
@@ -424,11 +428,12 @@ int nr_rasterize_backward_lights(const nrRasterConfig *cfg, const float *vertice
     a.grad_light = a.lights.num > 0 ? grad_light_data : nullptr;
     a.det_light = nullptr;
     a.det_verts = a.det_tex = a.det_vt = a.det_vn = nullptr;
-    a.det_scale = 4294967296.f;     // 2^32: resolution 2.3e-10, |sum| < 2.1e9
+    a.det_gmax = nullptr;
     if (cfg->flags & NR_DETERMINISTIC) {
         if (!deterministic_scratch || ((uintptr_t)deterministic_scratch & 7))
             return fail(NR_ERR_INVALID_ARGUMENT, "NR_DETERMINISTIC needs deterministic_scratch (8-byte aligned, zero-filled)");
         long long *p = (long long *)deterministic_scratch;
+        a.det_gmax = (unsigned *)(p + det_fixed_elems(cfg));
         a.det_verts = p;
         p += (size_t)cfg->batch * cfg->num_vertices * 3;
         if (grad_textures) {

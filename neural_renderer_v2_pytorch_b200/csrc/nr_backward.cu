@@ -187,16 +187,70 @@ __device__ __forceinline__ bool run_reduce(int key, bool valid, float (&v)[N], i
 // 16-pixel row segments of the tile, so the pixels of one face form runs in lane order.
 // Accumulate one contribution.  Float atomics (default) commute only up to rounding, so the result
 // depends on arrival order; in deterministic mode the value is rounded ONCE to 64-bit fixed point
-// (value * 2^k) and added with integer atomics, which are exactly associative: the sum is bit-identical
-// from run to run whatever the order.  The warp-level run sums in front of it have a fixed order.
+// (value * scale, scale = 2^(32 - E_b) of the view: det_scale) and added with integer atomics, which are exactly
+// associative: the sum is bit-identical from run to run whatever the order.  The warp-level run sums in front of it
+// have a fixed order.  A non-finite value goes to the float output instead: for NaN and +-inf alone the float sum
+// does not depend on the order either (NaN absorbs, +inf + -inf = NaN), and k_fixed_to_float adds onto it.
 template <bool DET, class Index>
-__device__ __forceinline__ void accumulate(float *dst_f, long long *dst_i, Index idx, float v, float scale) {
-    if (DET) {
+__device__ __forceinline__ void accumulate(float *dst_f, long long *dst_i, Index idx, float v, double scale) {
+    if (DET && isfinite(v)) {
         atomicAdd(reinterpret_cast<unsigned long long *>(dst_i + idx),
-                  (unsigned long long)__double2ll_rn((double)v * (double)scale));
+                  (unsigned long long)__double2ll_rn((double)v * scale));
     } else {
         atomicAdd(dst_f + idx, v);
     }
+}
+
+// 2^k as a double, k in [-1022, 1023]
+__device__ __forceinline__ double exp2i(int k) { return __hiloint2double((1023 + k) << 20, 0); }
+// E_b: frexp exponent of view b's max |grad_images| (max in [2^(E-1), 2^E)), 0 for an all-zero view
+__device__ __forceinline__ int det_exponent(const unsigned *gmax, int b) {
+    int e;
+    frexpf(__uint_as_float(gmax[b]), &e);
+    return e;
+}
+// Deterministic mode sums view b in units of 2^(E_b - 32): the resolution follows the size of the upstream
+// gradient (2^(E_b - 32) <= 4.7e-10 max |G|) and so does the range (|sum| < 2^(31 + E_b)).  Scaling a view's G by a
+// power of two scales its fixed-point words not at all and its gradients exactly; each view's bits depend on its
+// own G only, not on the batch it is rendered in.  The scale is a power of two, so v * scale is exact in double.
+__device__ __forceinline__ double det_scale(const unsigned *gmax, int b) { return exp2i(32 - det_exponent(gmax, b)); }
+
+// per-view max |G| over the finite values of grad_images [B, n] (n = C S S): grid = B * chunks blocks, atomicMax
+// on the bits of a non-negative float (ordered like the float, so the result does not depend on the order).  Each
+// thread keeps U loads in flight (float4 where the rows allow it): one load at a time left the kernel waiting on
+// DRAM latency at 0.6 TB/s.
+__device__ __forceinline__ float finite_absmax(float m, float x) { return isfinite(x) ? fmaxf(m, fabsf(x)) : m; }
+template <int U>
+__global__ void __launch_bounds__(256)
+k_det_gmax(const float *__restrict__ g, unsigned *__restrict__ gmax, long long n, int chunks) {
+    const int b = blockIdx.x / chunks, chunk = blockIdx.x - b * chunks;
+    const float *gb = g + (size_t)b * n;
+    const long long stride = (long long)chunks * blockDim.x, t = (long long)chunk * blockDim.x + threadIdx.x;
+    float m = 0.f;
+    if ((n & 3) == 0 && ((uintptr_t)g & 15) == 0) {
+        const float4 *g4 = reinterpret_cast<const float4 *>(gb);
+        const long long n4 = n >> 2;
+        for (long long i = t; i < n4; i += U * stride) {
+            float4 x[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u)
+                x[u] = i + u * stride < n4 ? __ldg(g4 + i + u * stride) : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+            for (int u = 0; u < U; ++u)
+                m = finite_absmax(finite_absmax(finite_absmax(finite_absmax(m, x[u].x), x[u].y), x[u].z), x[u].w);
+        }
+    } else {
+        for (long long i = t; i < n; i += U * stride) {
+            float x[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u) x[u] = i + u * stride < n ? __ldg(gb + i + u * stride) : 0.f;
+#pragma unroll
+            for (int u = 0; u < U; ++u) m = finite_absmax(m, x[u]);
+        }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, d));
+    if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(gmax + b, __float_as_uint(m));
 }
 
 // Gradient of the light data [L, B, 8] from one warp of one view b (autograd of rasterize.py:256-283 with respect
@@ -209,7 +263,7 @@ __device__ __forceinline__ void accumulate(float *dst_f, long long *dst_i, Index
 // at most 7 accumulations per (warp, light), never one per pixel.
 template <bool DET>
 __device__ __forceinline__ void light_param_grads(const BackwardArgs &a, int b, int lane, bool on, const float n[3],
-                                                  const float w[3]) {
+                                                  const float w[3], double dscale) {
     const LightArgs &L = a.lights;
     for (int l = 0; l < L.num; ++l) {
         const int type = __ldg(L.types + l);
@@ -252,7 +306,7 @@ __device__ __forceinline__ void light_param_grads(const BackwardArgs &a, int b, 
         for (int i = 1; i < 7; ++i)
             if (lane == i) v = p[i];
         const bool mine = lane < 3 || (lane < 6 && has_dir) || (lane == 6 && has_alpha);
-        if (mine && v != 0.f) accumulate<DET>(a.grad_light, a.det_light, o + lane, v, a.det_scale);
+        if (mine && v != 0.f) accumulate<DET>(a.grad_light, a.det_light, o + lane, v, dscale);
     }
 }
 
@@ -359,6 +413,7 @@ k_backward(const __grid_constant__ BackwardArgs a) {
     for (int work = blockIdx.x, it = 0; work < count; work += gridDim.x, ++it) {
     int b, tx, ty;
     tile_of(work, b, tx, ty);
+    const double dscale = DET ? det_scale(a.det_gmax, b) : 0.;    // set by k_det_gmax, which pdl_wait() waited for
     // item `it` is in stage s, its (it >> 1)-th use
     const int s = it & 1;
     const unsigned char *st = stage_smem + s * stage_bytes;
@@ -550,7 +605,7 @@ k_backward(const __grid_constant__ BackwardArgs a) {
 #pragma unroll
                         for (int c = 0; c < 3; ++c)
                             if (gn[c] != 0.f)
-                                accumulate<DET>(a.lights.grad_vnormals, a.det_vn, ovn + 3 * (size_t)vid[k] + c, q[k] * gn[c], a.det_scale);
+                                accumulate<DET>(a.lights.grad_vnormals, a.det_vn, ovn + 3 * (size_t)vid[k] + c, q[k] * gn[c], dscale);
                 }
                 if (LGRAD && lit) {
                     lg_on = true;
@@ -569,8 +624,8 @@ k_backward(const __grid_constant__ BackwardArgs a) {
                     const size_t o = (size_t)b * a.nvt * 2;
 #pragma unroll
                     for (int k = 0; k < 3; ++k) {
-                        if (gu[k] != 0.f) accumulate<DET>(a.grad_vt, a.det_vt, o + 2 * (size_t)tvid[k], gu[k], a.det_scale);
-                        if (gv[k] != 0.f) accumulate<DET>(a.grad_vt, a.det_vt, o + 2 * (size_t)tvid[k] + 1, gv[k], a.det_scale);
+                        if (gu[k] != 0.f) accumulate<DET>(a.grad_vt, a.det_vt, o + 2 * (size_t)tvid[k], gu[k], dscale);
+                        if (gv[k] != 0.f) accumulate<DET>(a.grad_vt, a.det_vt, o + 2 * (size_t)tvid[k] + 1, gv[k], dscale);
                     }
                 }
                 }   // tex_ok
@@ -613,9 +668,9 @@ k_backward(const __grid_constant__ BackwardArgs a) {
                     // one test per corner instead of one per component (every tested reduction costs a branch
                     // with a reconvergence barrier); z only moves where there is colour or depth to explain
                     if ((vg[3 * k] != 0.f) | (vg[3 * k + 1] != 0.f) | (vg[3 * k + 2] != 0.f)) {
-                        accumulate<DET>(pf, pi, 0, vg[3 * k], a.det_scale);
-                        accumulate<DET>(pf, pi, 1, vg[3 * k + 1], a.det_scale);
-                        if (has_z) accumulate<DET>(pf, pi, 2, vg[3 * k + 2], a.det_scale);
+                        accumulate<DET>(pf, pi, 0, vg[3 * k], dscale);
+                        accumulate<DET>(pf, pi, 1, vg[3 * k + 1], dscale);
+                        if (has_z) accumulate<DET>(pf, pi, 2, vg[3 * k + 2], dscale);
                     }
                 }
             }
@@ -635,21 +690,30 @@ k_backward(const __grid_constant__ BackwardArgs a) {
                     long long *pi = DET ? a.det_tex + o + tap[t] : nullptr;
 #pragma unroll
                     for (int c = 0; c < 3; ++c)
-                        accumulate<DET>(pf, pi, c * (int)T, tg[t * 3 + c], a.det_scale);
+                        accumulate<DET>(pf, pi, c * (int)T, tg[t * 3 + c], dscale);
                 }
             }
         }
     }
     // ---- light parameters: summed over the warp's 32 pixels, one accumulation per (warp, light, parameter)
     if (LIT && LGRAD && __ballot_sync(0xffffffffu, lg_on) != 0u)
-        light_param_grads<DET>(a, b, lane, lg_on, lg_n, lg_w);
+        light_param_grads<DET>(a, b, lane, lg_on, lg_n, lg_w, dscale);
     }   // tiles
 }
 
+// element i belongs to view (i / per_view) % B: per_view = the view's element count for [B, ...] gradients, 8 for the
+// light data [L, B, 8].  Added onto dst, which holds the non-finite contributions (and zeros elsewhere).
+// Grid: x over one view's elements, y strides over the outer index o = i / per_view (o < outer), so that no thread
+// divides an element index: view b = o % B.
 __global__ void __launch_bounds__(256)
-k_fixed_to_float(const long long *__restrict__ src, float *__restrict__ dst, size_t n, float inv_scale) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[i] += (float)((double)src[i] * (double)inv_scale);
+k_fixed_to_float(const long long *__restrict__ src, float *__restrict__ dst, size_t per_view, int outer, int B,
+                 const unsigned *__restrict__ gmax) {
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= per_view) return;
+    for (int o = blockIdx.y; o < outer; o += gridDim.y) {
+        const size_t i = (size_t)o * per_view + j;
+        dst[i] += (float)((double)src[i] * exp2i(det_exponent(gmax, o % B) - 32));
+    }
 }
 
 // Differentiation.backward on channels-last tensors (the public differentiation() op).
@@ -733,6 +797,14 @@ cudaError_t launch_backward(const BackwardArgs &args, cudaStream_t stream) {
     const long long tiles = (long long)a.ntx * a.ntx * a.B;
     // exactly the resident CTAs (4 per SM): a second wave of the static tile stride only adds a tail
     const int grid = (int)(tiles < (long long)a.sm_count * 4 ? tiles : (long long)a.sm_count * 4);
+    if (a.det_verts) {
+        // the per-view scales of the fixed-point sums, ahead of k_backward (its pdl_wait() waits for this kernel)
+        // one resident wave (8 blocks of 256 per SM), at least 16 k values per block
+        const long long n = (long long)a.C * a.S * a.S;
+        const long long want = (n + 16383) / 16384, cap = (long long)a.sm_count * 8 / a.B;
+        const int chunks = (int)(want < cap ? want : (cap > 1 ? cap : 1));
+        k_det_gmax<4><<<(unsigned)((long long)a.B * chunks), 256, 0, stream>>>(a.grad_images, a.det_gmax, n, chunks);
+    }
     ProfScope p(PROF_BACKWARD, stream);
     if (a.grad_light && a.lights.num > 0) {
         // light gradients: the lit variants with the light-parameter reduction (a.C does not matter: CT = 0)
@@ -770,15 +842,18 @@ cudaError_t launch_backward(const BackwardArgs &args, cudaStream_t stream) {
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess || !a.det_verts) return e;
     // fixed point -> float, added onto the caller's (zero-filled) gradient tensors
-    const float inv = 1.f / a.det_scale;
-    auto conv = [&](const long long *src, float *dst, size_t n) {
-        if (src && dst && n) k_fixed_to_float<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(src, dst, n, inv);
+    auto conv = [&](const long long *src, float *dst, size_t n, size_t per_view) {
+        if (src && dst && n) {     // n / per_view = B, or L * B for the light data
+            const int outer = (int)(n / per_view);
+            k_fixed_to_float<<<dim3((unsigned)((per_view + 255) / 256), (unsigned)(outer < 65535 ? outer : 65535)), 256, 0,
+                               stream>>>(src, dst, per_view, outer, a.B, a.det_gmax);
+        }
     };
-    conv(a.det_verts, a.grad_verts, (size_t)a.B * a.nv * 3);
-    conv(a.det_tex, a.grad_tex, (size_t)a.B * 3 * a.H * a.W);
-    conv(a.det_vt, a.grad_vt, (size_t)a.B * a.nvt * 2);
-    conv(a.det_vn, a.lights.grad_vnormals, (size_t)a.B * a.nv * 3);
-    conv(a.det_light, a.grad_light, (size_t)a.lights.num * a.B * 8);
+    conv(a.det_verts, a.grad_verts, (size_t)a.B * a.nv * 3, (size_t)a.nv * 3);
+    conv(a.det_tex, a.grad_tex, (size_t)a.B * 3 * a.H * a.W, (size_t)3 * a.H * a.W);
+    conv(a.det_vt, a.grad_vt, (size_t)a.B * a.nvt * 2, (size_t)a.nvt * 2);
+    conv(a.det_vn, a.lights.grad_vnormals, (size_t)a.B * a.nv * 3, (size_t)a.nv * 3);
+    conv(a.det_light, a.grad_light, (size_t)a.lights.num * a.B * 8, 8);
     return cudaGetLastError();
 }
 

@@ -99,9 +99,11 @@ struct BackwardArgs {
     int sm_count;
     float *grad_verts, *grad_tex, *grad_vt;
     // deterministic mode: 64-bit fixed-point accumulators (same shapes as the three gradients,
-    // laid out back to back) and the power-of-two scale; null = float atomics
+    // laid out back to back); null = float atomics
     long long *det_verts, *det_tex, *det_vt, *det_vn;   // det_vn: grad_vertex_normals (lights)
-    float det_scale;
+    // [B] max |grad_images| of each view over its finite values, as float bits (zero-filled, set by launch_backward):
+    // view b is summed in units of 2^(E_b - 32), E_b its frexp exponent.  Read by the DET variants only.
+    unsigned *det_gmax;
     LightArgs lights;
     int B, nv, nf, R, S, ntx, C, flags, nvt, H, W;
     int face_stride;        // ints between the face (and texture-face) rows of consecutive views: 3 nf or 0

@@ -14,7 +14,8 @@ class RasterizeHyperparam:
         self.draw_rgb = draw_rgb
         self.draw_silhouettes = draw_silhouettes
         self.draw_depth = draw_depth
-        # not in the reference: bit-reproducible gradients (fixed-point accumulation, see nr_b200.h)
+        # not in the reference: bit-reproducible gradients (fixed-point sums in a unit chosen per view from its
+        # max |grad_images|: exact under power-of-two loss scaling, NaN / inf as in float mode; see nr_b200.h)
         self.deterministic = False
 
 

@@ -219,12 +219,14 @@ def test_specular_alpha_where_the_base_is_zero(nr):
         grad_close(P[k].grad.cpu().numpy(), want[k], k)
 
 
+@pytest.mark.parametrize("k", [-26, 0, 24])
 @pytest.mark.parametrize("deterministic", [False, True])
-def test_full_size_ambient_colour_gradient(nr, deterministic):
+def test_full_size_ambient_colour_gradient(nr, deterministic, k):
     """Teapot, 64 views at 512^2, RGB, one ambient light: the image is linear in its colour, so
     d loss / d colour[b, c] = sum G * image_unlit[b, c] (float64 sum of an unlit render of the same inputs).  Every
     foreground pixel of a view adds to the same 3 values: the reduction at full contention.  G is uniform in [0, 1)
-    so that the sum is well conditioned and the bar measures the reduction, not float32 cancellation."""
+    so that the sum is well conditioned and the bar measures the reduction, not float32 cancellation.  G is scaled
+    by 2^k: 2^-26 is a mean loss over config 2's image, 2^24 a loss scaler's factor that puts the sums past 2^31."""
     import bench
     dev = torch.device("cuda:0")
     w = dict(bench.WORKLOADS["cfg2"], mode="rgb")
@@ -232,7 +234,7 @@ def test_full_size_ambient_colour_gradient(nr, deterministic):
     B, S = w["views"], w["S"]
     v, faces = inp["vertices"].to(dev), inp["faces"].to(dev)
     vt, ft, tex = inp["vt"].to(dev), inp["ft"].to(dev), inp["textures"].to(dev)
-    G = torch.rand((B, 3, S, S), generator=torch.Generator().manual_seed(5)).to(dev)
+    G = (torch.rand((B, 3, S, S), generator=torch.Generator().manual_seed(5)) * 2.0 ** k).to(dev)
 
     def hp():
         h = nr.RasterizeHyperparam(image_size=S, anti_aliasing=False)
@@ -245,6 +247,8 @@ def test_full_size_ambient_colour_gradient(nr, deterministic):
     img = nr.rasterize_rgb(v, faces, p, hp())
     (img * G).sum().backward()
     want = (G.double() * unlit.double()).sum(dim=(2, 3))
+    if k == 24:
+        assert float(want.abs().max()) > 2.0 ** 31
     np.testing.assert_allclose(color.grad.double().cpu().numpy(), want.cpu().numpy(), rtol=1e-5)
 
 

@@ -79,6 +79,12 @@ enum {
                                  NR_DRAW_RGB, `faces_textures` is [B, nf, 3] as well; view b reads row b of both.
                                  Views with fewer faces pad their rows with a degenerate face (three equal indices,
                                  e.g. 0 0 0): it is never drawn and gets no gradient.  faces must not be NULL. */
+#define NR_FACE_TEXTURES 2048 /* forward and backward, with NR_DRAW_RGB: per-face texture cubes, the texture format of
+                                 the v1 renderer and of Mesh.  `textures` is [B, nf, ts, ts, ts, 3] (channels last);
+                                 face f of view b samples textures[b, f] trilinearly at t_k = q_k (ts-1) depth / z_k
+                                 (clamped to [0, ts-1-eps]; DESIGN.md "API notes").  vertices_textures, faces_textures,
+                                 grad_vertices_textures and aux_map must be NULL; tex_height = tex_width = ts >= 1,
+                                 num_tex_vertices = 0, nf * ts^3 * 3 < 2^31.  grad_textures has the textures' shape. */
 
 /* Mirrors RasterizeHyperparam (rasterize_param.py:13-33) plus the tensor extents. */
 typedef struct nrRasterConfig {
@@ -192,7 +198,9 @@ NR_API size_t nr_workspace_bytes(const nrRasterConfig *cfg, int64_t pair_capacit
  *                                    [B, nf, 3] with NR_VIEW_FACES
  *   vertices_textures   [B, nvt, 2]  texel coordinates           (NR_DRAW_RGB only)
  *   faces_textures      [nf, 3]      ids into vertices_textures  (NR_DRAW_RGB only; [B, nf, 3] with NR_VIEW_FACES)
- *   textures            [B, 3, H, W]                             (NR_DRAW_RGB only)
+ *   textures            [B, 3, H, W]                             (NR_DRAW_RGB only; [B, nf, ts, ts, ts, 3] with
+ *                                                                 NR_FACE_TEXTURES, then vertices_textures and
+ *                                                                 faces_textures are NULL)
  *   face_index_map      [B, R, R]    out, -1 on background (never NULL)
  *   weight_map          [B, R, R, 3] out, optional (NULL to skip)
  *   depth_map           [B, R, R]    out, optional (NULL to skip); 1/sum(w/z), 0 on background
@@ -242,7 +250,7 @@ NR_API int nr_rasterize_forward(const nrRasterConfig *cfg, const float *vertices
  *   tile_list           from the forward, or NULL (then every tile is visited)
  *   grad_images         [B, C, S, S] upstream gradient
  *   grad_vertices       [B, nv, 3]   out, ACCUMULATED into (caller zero-fills)
- *   grad_textures       [B, 3, H, W] out, accumulated, optional
+ *   grad_textures       [B, 3, H, W] out, accumulated, optional ([B, nf, ts, ts, ts, 3] with NR_FACE_TEXTURES)
  *   grad_vertices_textures [B, nvt, 2] out, accumulated, optional
  *   deterministic_scratch  only with NR_DETERMINISTIC in cfg->flags: nr_deterministic_scratch_bytes(cfg)
  *                       zero-filled bytes.  Contributions are then rounded once to 64-bit fixed point

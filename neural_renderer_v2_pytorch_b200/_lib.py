@@ -28,6 +28,7 @@ NR_SPARSE_MAPS = 128
 NR_FINE_TILES = 256
 NR_DENSE_RASTER = 512
 NR_VIEW_FACES = 1024
+NR_FACE_TEXTURES = 2048
 
 # every symbol include/nr_b200.h declares (tests/test_abi.py checks header <-> library <-> this list)
 SYMBOLS = (

@@ -126,6 +126,15 @@ int view_face_stride(const nrRasterConfig *cfg) {
     return (cfg->flags & NR_VIEW_FACES) ? 3 * cfg->num_faces : 0;
 }
 
+// texture elements of one view: [3, H, W], or with NR_FACE_TEXTURES the per-face cubes [nf, ts, ts, ts, 3] (H = W = ts)
+size_t tex_elems_per_view(const nrRasterConfig *cfg) {
+    if (cfg->flags & NR_FACE_TEXTURES) {
+        const size_t ts = cfg->tex_height > 0 ? (size_t)cfg->tex_height : 0;
+        return (size_t)(cfg->num_faces > 0 ? cfg->num_faces : 0) * ts * ts * ts * 3;
+    }
+    return (size_t)3 * cfg->tex_height * cfg->tex_width;
+}
+
 int check_config(const nrRasterConfig *cfg) {
     if (!cfg) return fail(NR_ERR_INVALID_ARGUMENT, "config is NULL");
     if (cfg->batch < 0 || cfg->num_vertices < 0 || cfg->num_faces < 0 || cfg->image_size <= 0)
@@ -137,6 +146,15 @@ int check_config(const nrRasterConfig *cfg) {
     if (R > 32768) return fail(NR_ERR_INVALID_ARGUMENT, "internal resolution > 32768");
     if (!(cfg->flags & (NR_DRAW_RGB | NR_DRAW_SILHOUETTES | NR_DRAW_DEPTH)))
         return fail(NR_ERR_INVALID_ARGUMENT, "nothing to draw: no NR_DRAW_* flag");
+    if (cfg->flags & NR_FACE_TEXTURES) {
+        if (!(cfg->flags & NR_DRAW_RGB)) return fail(NR_ERR_INVALID_ARGUMENT, "NR_FACE_TEXTURES needs NR_DRAW_RGB");
+        if (cfg->tex_height < 1 || cfg->tex_width != cfg->tex_height || cfg->num_tex_vertices != 0)
+            return fail(NR_ERR_INVALID_ARGUMENT, "NR_FACE_TEXTURES needs tex_height = tex_width = ts >= 1 and num_tex_vertices = 0");
+        // the kernels address a view's cubes with 32-bit offsets
+        const long long ts = cfg->tex_height;
+        if (ts > 1290 || (long long)cfg->num_faces * ts * ts * ts * 3 >= (1ll << 31))
+            return fail(NR_ERR_INVALID_ARGUMENT, "NR_FACE_TEXTURES: nf * ts^3 * 3 of one view must be below 2^31");
+    }
     return NR_OK;
 }
 
@@ -203,7 +221,7 @@ int nr_event_synchronize(void *event) {
 // back to back.  The B per-view maxima of |grad_images| (BackwardArgs::det_gmax) follow them.
 static size_t det_fixed_elems(const nrRasterConfig *cfg) {
     return (size_t)cfg->batch * cfg->num_vertices * 3 +
-           (size_t)cfg->batch * 3 * cfg->tex_height * cfg->tex_width +
+           (size_t)cfg->batch * tex_elems_per_view(cfg) +
            (size_t)cfg->batch * cfg->num_tex_vertices * 2 +
            (size_t)cfg->batch * cfg->num_vertices * 3;
 }
@@ -234,9 +252,13 @@ int nr_rasterize_forward(const nrRasterConfig *cfg, const float *vertices, const
     if (!vertices && cfg->batch * cfg->num_faces > 0) return fail(NR_ERR_INVALID_ARGUMENT, "vertices is NULL");
     if (!face_index_map) return fail(NR_ERR_INVALID_ARGUMENT, "face_index_map is NULL");
     if ((cfg->flags & NR_VIEW_FACES) && !faces) return fail(NR_ERR_INVALID_ARGUMENT, "NR_VIEW_FACES needs faces [B, nf, 3]");
-    if (rgb && (!vertices_textures || !faces_textures || !textures))
+    const bool cube = (cfg->flags & NR_FACE_TEXTURES) != 0;
+    if (cube && (vertices_textures || faces_textures || !textures))
+        return fail(NR_ERR_INVALID_ARGUMENT, "NR_FACE_TEXTURES needs textures [B, nf, ts, ts, ts, 3] and NULL vertices_textures / faces_textures");
+    if (cube && aux_map) return fail(NR_ERR_INVALID_ARGUMENT, "NR_FACE_TEXTURES: no aux_map in this mode");
+    if (rgb && !cube && (!vertices_textures || !faces_textures || !textures))
         return fail(NR_ERR_INVALID_ARGUMENT, "NR_DRAW_RGB needs vertices_textures, faces_textures and textures");
-    if (rgb && (cfg->tex_height <= 0 || cfg->tex_width <= 0 || cfg->num_tex_vertices <= 0))
+    if (rgb && !cube && (cfg->tex_height <= 0 || cfg->tex_width <= 0 || cfg->num_tex_vertices <= 0))
         return fail(NR_ERR_INVALID_ARGUMENT, "NR_DRAW_RGB needs positive texture extents");
     if (images && aa && !images_internal)
         return fail(NR_ERR_INVALID_ARGUMENT, "anti-aliasing needs images_internal");
@@ -398,7 +420,11 @@ int nr_rasterize_backward_lights(const nrRasterConfig *cfg, const float *vertice
     if (!vertices || !face_index_map || !images_internal || !grad_images || !grad_vertices)
         return fail(NR_ERR_INVALID_ARGUMENT, "backward: a required pointer is NULL");
     if ((cfg->flags & NR_VIEW_FACES) && !faces) return fail(NR_ERR_INVALID_ARGUMENT, "NR_VIEW_FACES needs faces [B, nf, 3]");
-    if (rgb && (!vertices_textures || !faces_textures || !textures))
+    const bool cube = (cfg->flags & NR_FACE_TEXTURES) != 0;
+    if (cube && (vertices_textures || faces_textures || grad_vertices_textures || !textures))
+        return fail(NR_ERR_INVALID_ARGUMENT, "NR_FACE_TEXTURES needs textures [B, nf, ts, ts, ts, 3] and NULL vertices_textures / faces_textures");
+    if (cube && aux_map) return fail(NR_ERR_INVALID_ARGUMENT, "NR_FACE_TEXTURES: no aux_map in this mode");
+    if (rgb && !cube && (!vertices_textures || !faces_textures || !textures))
         return fail(NR_ERR_INVALID_ARGUMENT, "NR_DRAW_RGB needs vertices_textures, faces_textures and textures");
     if (cfg->batch == 0) return NR_OK;
     nr::BackwardArgs a;
@@ -438,7 +464,7 @@ int nr_rasterize_backward_lights(const nrRasterConfig *cfg, const float *vertice
         p += (size_t)cfg->batch * cfg->num_vertices * 3;
         if (grad_textures) {
             a.det_tex = p;
-            p += (size_t)cfg->batch * 3 * cfg->tex_height * cfg->tex_width;
+            p += (size_t)cfg->batch * tex_elems_per_view(cfg);
         }
         if (grad_vertices_textures) {
             a.det_vt = p;

@@ -155,6 +155,66 @@ __device__ __forceinline__ void sample_texture_backward(const float *__restrict_
     }
 }
 
+// Backward of sample_face_texture() (per-face texture cubes): the 8 tap offsets (float index of channel 0 within the
+// view's [nf, ts, ts, ts, 3] textures, -1 when the tap reads as zero) and weights, and the gradient w.r.t. the face
+// depths through zz and depth.  g_lit / cw / g / rgb_tex as in sample_texture_backward; cell = face * ts^3 + base
+// texel (equal cell => equal taps).  d rgb / d t_k = sum_taps (c_k ? +1 : -1) prod_{j != k} w_j texel; the clamp
+// passes the gradient on [0, hi] (torch.clamp), floor passes none.
+__device__ __forceinline__ void sample_face_texture_backward(const float *__restrict__ tex_b, int f, int ts, float eps,
+                                                             const float q[3], const float z[3], const float g_lit[3],
+                                                             const float cw[3], float g[3], float rgb_tex[3], int tap[8],
+                                                             float tw[8], int &cell, float gz[3]) {
+    const CubeCoord cc = cube_coord(q, z, ts, eps);
+    const float hi = fmaxf(__fsub_rn((float)(ts - 1), eps), 0.f);
+    int i[3];
+    float fr[3], lo[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const float fl = floorf(cc.t[k]);
+        i[k] = (int)fl;
+        fr[k] = __fsub_rn(cc.t[k], fl);
+        lo[k] = __fsub_rn(1.f, fr[k]);
+    }
+    const int base = (f * ts + i[0]) * ts * ts + i[1] * ts + i[2];
+    cell = base;
+    g[0] = g_lit[0] * cw[0]; g[1] = g_lit[1] * cw[1]; g[2] = g_lit[2] * cw[2];
+    rgb_tex[0] = rgb_tex[1] = rgb_tex[2] = 0.f;
+    float gt[3] = {0.f, 0.f, 0.f};      // d loss / d t_k
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+        const int c0 = c >> 2, c1 = (c >> 1) & 1, c2 = c & 1;
+        const float w0 = c0 ? fr[0] : lo[0], w1 = c1 ? fr[1] : lo[1], w2 = c2 ? fr[2] : lo[2];
+        tw[c] = w0 * w1 * w2;
+        tap[c] = -1;
+        if (i[0] + c0 >= ts || i[1] + c1 >= ts || i[2] + c2 >= ts) continue;
+        tap[c] = (base + (c0 * ts + c1) * ts + c2) * 3;
+        const float *pt = tex_b + tap[c];
+        float d = 0.f;
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) {
+            const float tv = __ldg(pt + ch);
+            d += g[ch] * tv;
+            rgb_tex[ch] += tw[c] * tv;
+        }
+        gt[0] += (c0 ? d : -d) * (w1 * w2);
+        gt[1] += (c1 ? d : -d) * (w0 * w2);
+        gt[2] += (c2 ? d : -d) * (w0 * w1);
+    }
+    // t_k = s_k depth, s_k = q_k (ts - 1) / zz_k, depth = 1 / sum_j (q_j / zz_j + 1e-10)
+    float P = 0.f;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        if (!(cc.t0[k] >= 0.f && cc.t0[k] <= hi)) gt[k] = 0.f;
+        P += gt[k] * cc.s[k];
+    }
+    const float dd = P * cc.depth * cc.depth;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const float iz = 1.f / cc.zz[k];
+        gz[k] = (dd * q[k] * iz - gt[k] * cc.s[k] * cc.depth) * iz;
+    }
+}
+
 // Warp-level segmented sum over runs of equal `key` in lane order (a warp is one image row
 // segment, so the pixels of one face / one texel cell form runs).  Afterwards the LAST lane of
 // every run holds the run total in v[]; returns true on those lanes.  Fixed summation order.
@@ -373,7 +433,8 @@ __device__ __forceinline__ float ld_stencil(const float *p) {
 // that calls with constant lights run exactly the code they ran before light gradients existed.
 // STAGED: the face indices and the stencil operands come from shared memory (staged front above); otherwise from
 // global memory (any R, any alignment; NR_FORCE_UNSTAGED_BACKWARD=1).  Both compute bit-identical results.
-template <int CT, bool NEED_UV, bool DET, bool AUX, bool LGRAD = false, bool STAGED = false>
+// TEX: the texture kind; per-face cubes (NR_FACE_TEXTURES) only in the generic variants (CT = 0, no aux map, no uv).
+template <int CT, bool NEED_UV, bool DET, bool AUX, bool LGRAD = false, bool STAGED = false, int TEX = TEX_UV>
 __global__ void __launch_bounds__(TILE_THREADS, 4)
 k_backward(const __grid_constant__ BackwardArgs a) {
     extern __shared__ __align__(128) unsigned char stage_smem[];
@@ -509,8 +570,14 @@ k_backward(const __grid_constant__ BackwardArgs a) {
     // ---- per-pixel contributions
     int vid[3] = {0, 0, 0};
     float vg[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};   // (x, y, z) gradient of the 3 corners
-    float tg[12] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};   // 4 taps x rgb
-    int tap[4] = {-1, -1, -1, -1};
+    constexpr bool CUBE = TEX == TEX_CUBE;
+    constexpr int NTAP = CUBE ? 8 : 4;     // bilinear or trilinear taps
+    float tg[NTAP * 3];                    // taps x rgb
+#pragma unroll
+    for (int i = 0; i < NTAP * 3; ++i) tg[i] = 0.f;
+    int tap[NTAP];
+#pragma unroll
+    for (int t = 0; t < NTAP; ++t) tap[t] = -1;
     int cell = 0;
     bool has_tex = false;
     // light-parameter gradients: the interpolated normal and d loss / d colour weight of a lit pixel, kept
@@ -564,11 +631,12 @@ k_backward(const __grid_constant__ BackwardArgs a) {
         if (rgb) {
             const float g_lit[3] = {gcen[0], gcen[1], gcen[2]};
             if (g_lit[0] != 0.f || g_lit[1] != 0.f || g_lit[2] != 0.f) {
-                const int32_t *fti = a.ft + frow;
-                const float *vtb = a.vt + (size_t)b * a.nvt * 2;
                 int tvid[3];
                 float u[3], v[3];
                 bool tex_ok = true;      // an out-of-range texture-vertex index contributes nothing (the forward drew black)
+                if constexpr (!CUBE) {
+                const int32_t *fti = a.ft + frow;
+                const float *vtb = a.vt + (size_t)b * a.nvt * 2;
 #pragma unroll
                 for (int k = 0; k < 3; ++k) {
                     tvid[k] = __ldg(fti + k);
@@ -579,8 +647,9 @@ k_backward(const __grid_constant__ BackwardArgs a) {
                     u[k] = uv.x;
                     v[k] = uv.y;
                 }
+                }   // !CUBE
                 if (tex_ok) {
-                float gu[3] = {0.f, 0.f, 0.f}, gv[3] = {0.f, 0.f, 0.f}, tw[4], g[3], rgb_tex[3];
+                float gu[3] = {0.f, 0.f, 0.f}, gv[3] = {0.f, 0.f, 0.f}, tw[NTAP], g[3], rgb_tex[3];
                 float cw[3] = {1.f, 1.f, 1.f}, nrm[3] = {0.f, 0.f, 0.f};
                 const bool lit = LIT && a.lights.num > 0;
                 if (lit) {
@@ -592,6 +661,10 @@ k_backward(const __grid_constant__ BackwardArgs a) {
                             nrm[c] = __fadd_rn(nrm[c], __fmul_rn(q[k], __ldg(vnb + 3 * (size_t)vid[k] + c)));
                     light_weights(a.lights, b, a.B, nrm, cw, nullptr, nullptr);
                 }
+                if constexpr (CUBE)
+                    sample_face_texture_backward(a.tex + (size_t)b * a.nf * a.H * a.H * a.H * 3, f, a.H, a.eps, q, Z, g_lit,
+                                                 cw, g, rgb_tex, tap, tw, cell, gz);
+                else
                 sample_texture_backward<NEED_UV>(a.tex + (size_t)b * 3 * a.H * a.W, a.H, a.W, a.eps, q, Z, u, v, AUX ? tcs : nullptr,
                                         g_lit, cw, g, rgb_tex, tap, tw, cell, gz, gu, gv);
                 if (lit && a.lights.grad_vnormals) {
@@ -617,7 +690,7 @@ k_backward(const __grid_constant__ BackwardArgs a) {
                 }
                 has_tex = true;
 #pragma unroll
-                for (int t = 0; t < 4; ++t)
+                for (int t = 0; t < NTAP; ++t)
 #pragma unroll
                     for (int c = 0; c < 3; ++c) tg[t * 3 + c] = tw[t] * g[c];
                 if (NEED_UV) {
@@ -680,7 +753,21 @@ k_backward(const __grid_constant__ BackwardArgs a) {
     if (rgb && a.grad_tex) {
         const bool has = has_tex;
         if (__ballot_sync(0xffffffffu, has) != 0u) {
-            const bool tail = run_reduce<12>(cell, has, tg, lane);
+            const bool tail = run_reduce<NTAP * 3>(cell, has, tg, lane);
+            if constexpr (CUBE) {
+                // channels last: the three channels of a texel are adjacent
+                if (tail && has) {
+                    const size_t o = (size_t)b * a.nf * a.H * a.H * a.H * 3;
+#pragma unroll
+                    for (int t = 0; t < NTAP; ++t) {
+                        if (tap[t] < 0) continue;
+                        float *pf = a.grad_tex + o + tap[t];
+                        long long *pi = DET ? a.det_tex + o + tap[t] : nullptr;
+#pragma unroll
+                        for (int c = 0; c < 3; ++c) accumulate<DET>(pf, pi, c, tg[t * 3 + c], dscale);
+                    }
+                }
+            } else
             if (tail && has) {
                 const size_t T = (size_t)a.H * a.W, o = (size_t)b * 3 * T;
 #pragma unroll
@@ -777,14 +864,14 @@ static bool prepare_staging(BackwardArgs &s) {
                       aa ? ST_W_AA : ST_W, aa ? ST_H_AA : ST_H, s.C);
 }
 
-template <int CT, bool NEED_UV, bool DET, bool AUX, bool LGRAD = false>
+template <int CT, bool NEED_UV, bool DET, bool AUX, bool LGRAD = false, int TEX = TEX_UV>
 static void launch_variant(const BackwardArgs &a, bool staged, int grid, cudaStream_t stream) {
     const long long px = (long long)a.B * a.R * a.R;
     if (staged)
-        launch_after(2, px, k_backward<CT, NEED_UV, DET, AUX, LGRAD, true>, dim3(grid), dim3(TILE_THREADS),
+        launch_after(2, px, k_backward<CT, NEED_UV, DET, AUX, LGRAD, true, TEX>, dim3(grid), dim3(TILE_THREADS),
                      (size_t)st_smem_bytes(a.C, (a.flags & FLAG_AA) != 0), stream, a);
     else
-        launch_after(2, px, k_backward<CT, NEED_UV, DET, AUX, LGRAD, false>, dim3(grid), dim3(TILE_THREADS), 0, stream, a);
+        launch_after(2, px, k_backward<CT, NEED_UV, DET, AUX, LGRAD, false, TEX>, dim3(grid), dim3(TILE_THREADS), 0, stream, a);
 }
 
 cudaError_t launch_backward(const BackwardArgs &args, cudaStream_t stream) {
@@ -806,7 +893,17 @@ cudaError_t launch_backward(const BackwardArgs &args, cudaStream_t stream) {
         k_det_gmax<4><<<(unsigned)((long long)a.B * chunks), 256, 0, stream>>>(a.grad_images, a.det_gmax, n, chunks);
     }
     ProfScope p(PROF_BACKWARD, stream);
-    if (a.grad_light && a.lights.num > 0) {
+    if (a.flags & FLAG_FACE_TEX) {
+        // per-face texture cubes: generic variants, no uv gradient, no aux map (the C ABI refuses one)
+        const bool lgrad = a.grad_light && a.lights.num > 0;
+        if (a.det_verts) {
+            if (lgrad) launch_variant<0, false, true, false, true, TEX_CUBE>(a, staged, grid, stream);
+            else launch_variant<0, false, true, false, false, TEX_CUBE>(a, staged, grid, stream);
+        } else {
+            if (lgrad) launch_variant<0, false, false, false, true, TEX_CUBE>(a, staged, grid, stream);
+            else launch_variant<0, false, false, false, false, TEX_CUBE>(a, staged, grid, stream);
+        }
+    } else if (a.grad_light && a.lights.num > 0) {
         // light gradients: the lit variants with the light-parameter reduction (a.C does not matter: CT = 0)
         if (a.det_verts) {
             if (a.grad_vt) launch_variant<0, true, true, false, true>(a, staged, grid, stream);
@@ -850,7 +947,9 @@ cudaError_t launch_backward(const BackwardArgs &args, cudaStream_t stream) {
         }
     };
     conv(a.det_verts, a.grad_verts, (size_t)a.B * a.nv * 3, (size_t)a.nv * 3);
-    conv(a.det_tex, a.grad_tex, (size_t)a.B * 3 * a.H * a.W, (size_t)3 * a.H * a.W);
+    // textures per view: [3, H, W], or [nf, ts, ts, ts, 3] per-face cubes (H = W = ts)
+    const size_t tex_view = (a.flags & FLAG_FACE_TEX) ? (size_t)a.nf * a.H * a.H * a.H * 3 : (size_t)3 * a.H * a.W;
+    conv(a.det_tex, a.grad_tex, (size_t)a.B * tex_view, tex_view);
     conv(a.det_vt, a.grad_vt, (size_t)a.B * a.nvt * 2, (size_t)a.nvt * 2);
     conv(a.det_vn, a.lights.grad_vnormals, (size_t)a.B * a.nv * 3, (size_t)a.nv * 3);
     conv(a.det_light, a.grad_light, (size_t)a.lights.num * a.B * 8, 8);

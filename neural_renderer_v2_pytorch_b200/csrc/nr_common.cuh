@@ -18,7 +18,10 @@ constexpr int WARP_BH = 4;
 
 // nrRasterConfig.flags (include/nr_b200.h)
 constexpr int FLAG_RGB = 1, FLAG_SIL = 2, FLAG_DEPTH = 4, FLAG_BACKSIDE = 8, FLAG_AA = 16,
-              FLAG_DETERMINISTIC = 32;
+              FLAG_DETERMINISTIC = 32, FLAG_FACE_TEX = 2048;
+// Texture kind of the shading code, a template argument: UV textures [B, 3, H, W] (the reference's), or one
+// ts^3 RGB cube per face [B, nf, ts, ts, ts, 3] (NR_FACE_TEXTURES, the v1 format of Mesh)
+enum TexKind : int { TEX_UV = 0, TEX_CUBE = 1 };
 // Dense meshes (hundreds of faces per 16x16 tile) are binned into 8x8 tiles instead: four times shorter
 // lists to sort and to walk (general binning path and the FINE raster variants only).
 constexpr int FINE_TILE = 8;
@@ -287,6 +290,35 @@ __device__ __forceinline__ TexCoord texel_coord_stored(float depth, float nx, fl
     t.xf = fminf(fmaxf(t.x0, fminf(u[0], fminf(u[1], u[2]))), __fsub_rn(fmaxf(u[0], fmaxf(u[1], u[2])), eps));
     t.yf = fminf(fmaxf(t.y0, fminf(v[0], fminf(v[1], v[2]))), __fsub_rn(fmaxf(v[0], fmaxf(v[1], v[2])), eps));
     return t;
+}
+
+// Per-face texture cubes (NR_FACE_TEXTURES, textures [B, nf, ts, ts, ts, 3]): the cube coordinate of a foreground
+// pixel.  Axis k of the cube belongs to face corner k; t_k = (q_k (ts - 1) / zz_k) depth with the same regularised
+// depth as texel_coord(), clamped to [0, max(ts - 1 - eps, 0)].  Forward and backward both call this, so they agree
+// on the cell a pixel samples.
+struct CubeCoord {
+    float depth;
+    float s[3];            // q_k (ts - 1) / zz_k
+    float t0[3], t[3];     // before / after the clamp
+    float zz[3];           // z + 1e-10
+};
+__device__ __forceinline__ CubeCoord cube_coord(const float q[3], const float z[3], int ts, float eps) {
+    CubeCoord c;
+    const float n = (float)(ts - 1), hi = fmaxf(__fsub_rn(n, eps), 0.f);
+    float a[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        c.zz[k] = __fadd_rn(z[k], 1e-10f);
+        a[k] = __fadd_rn(__fdiv_rn(q[k], c.zz[k]), 1e-10f);
+    }
+    c.depth = __fdiv_rn(1.f, __fadd_rn(__fadd_rn(a[0], a[1]), a[2]));
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        c.s[k] = __fdiv_rn(__fmul_rn(q[k], n), c.zz[k]);
+        c.t0[k] = __fmul_rn(c.s[k], c.depth);
+        c.t[k] = fminf(fmaxf(c.t0[k], 0.f), hi);       // (NaN -> 0)
+    }
+    return c;
 }
 
 // Lights as the kernels see them (include/nr_b200.h: nrLights).

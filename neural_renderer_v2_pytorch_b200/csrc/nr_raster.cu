@@ -114,8 +114,8 @@ __device__ __forceinline__ bool edge_inside(float xp, float yp, const float4 &A,
 // Variants: RGB (texture sampling), AA (2x2 mean epilogue), FULL (everything optional: lights,
 // backgrounds, the weight / depth maps of rasterize_maps, resolutions that are no multiple of 16).
 // The plain variants leave that code out, which halves their size: at 75 KB the one-size kernel spent
-// as many issue slots waiting for instructions as for memory.
-template <bool RGB, bool AA, bool FULL, bool FINE>
+// as many issue slots waiting for instructions as for memory.  TEX: the texture kind (per-face cubes: FULL only).
+template <bool RGB, bool AA, bool FULL, bool FINE, int TEX = TEX_UV>
 __global__ void __launch_bounds__(TILE_THREADS, 4)
 k_raster(const RasterArgs a) {
     pdl_wait();         // the binning kernel's records, lists and header (nr_kernels.h)
@@ -338,7 +338,7 @@ k_raster(const RasterArgs a) {
             const int yh = yi + h * HALF_H, best = h ? z_l.best : z_u.best;
             float bw0 = 0.f, bw1 = 0.f, bw2 = 0.f, bz0 = 0.f, bz1 = 0.f, bz2 = 0.f;
             if (best >= 0) winner_weights(rec_b, best, xp, h ? yp_l : yp_u, bw0, bw1, bw2, bz0, bz1, bz2);
-            shade_block<RGB, AA, FULL>(a, b, xi, yh, (xi < R) && (yh < R), best, bw0, bw1, bw2, bz0, bz1, bz2, has_bg);
+            shade_block<RGB, AA, FULL, TEX>(a, b, xi, yh, (xi < R) && (yh < R), best, bw0, bw1, bw2, bz0, bz1, bz2, has_bg);
         }
     }   // items of this claim
     }   // claims
@@ -389,6 +389,16 @@ cudaError_t launch_raster(const RasterArgs &a, cudaStream_t stream) {
     const bool full = a.lights.num > 0 || a.lights.backgrounds || a.wmap || a.dmap || !a.images || (a.R & 15) ||
                       (rgb && a.face_stride != 0);
     ProfScope p(PROF_RASTER, stream);
+    if (a.flags & FLAG_FACE_TEX) {     // per-face texture cubes: colour, full-featured variants of their own
+        const long long px = (long long)a.B * a.R * a.R;
+        switch ((aa ? 1 : 0) | (a.fine ? 2 : 0)) {
+            case 0: launch_after(1, px, k_raster<true, false, true, false, TEX_CUBE>, dim3(grid), dim3(TILE_THREADS), 0, stream, a); break;
+            case 1: launch_after(1, px, k_raster<true, true, true, false, TEX_CUBE>, dim3(grid), dim3(TILE_THREADS), 0, stream, a); break;
+            case 2: launch_after(1, px, k_raster<true, false, true, true, TEX_CUBE>, dim3(grid), dim3(TILE_THREADS), 0, stream, a); break;
+            default: launch_after(1, px, k_raster<true, true, true, true, TEX_CUBE>, dim3(grid), dim3(TILE_THREADS), 0, stream, a); break;
+        }
+        return cudaGetLastError();
+    }
     if (a.fine) {       // dense meshes: the full-featured kernels over 8x8 tiles
         switch ((rgb ? 1 : 0) | (aa ? 2 : 0)) {
             case 0: launch_after(1, (long long)a.B * a.R * a.R, k_raster<false, false, true, true>, dim3(grid), dim3(TILE_THREADS), 0, stream, a); break;

@@ -905,7 +905,7 @@ k_zb_resolve(const RasterArgs a, long long words) {
 }
 
 // ---------------------------------------------------------------------------------------------- pass 5
-template <bool RGB, bool AA, bool FULL>
+template <bool RGB, bool AA, bool FULL, int TEX = TEX_UV>
 __global__ void __launch_bounds__(TILE_THREADS)
 k_zb_shade(const RasterArgs a) {
     pdl_wait();
@@ -946,7 +946,7 @@ k_zb_shade(const RasterArgs a) {
         bz0 = __ldg(vb + 3 * (size_t)i0 + 2); bz1 = __ldg(vb + 3 * (size_t)i1 + 2); bz2 = __ldg(vb + 3 * (size_t)i2 + 2);
         raw_weights(grid.center(xi), grid.center(yi), x0, y0, x1, y1, x2, y2, bw0, bw1, bw2);
     }
-    shade_block<RGB, AA, FULL>(a, b, xi, yi, valid, best, bw0, bw1, bw2, bz0, bz1, bz2, has_bg);
+    shade_block<RGB, AA, FULL, TEX>(a, b, xi, yi, valid, best, bw0, bw1, bw2, bz0, bz1, bz2, has_bg);
     // the backward walks the non-empty tiles only
     const int any = __syncthreads_or(best >= 0);
     if (any && tid == 0) {
@@ -992,7 +992,10 @@ cudaError_t launch_raster_zbuf(const RasterArgs &a, cudaStream_t stream) {
     const unsigned tiles = (unsigned)((long long)a.B * a.ntx * a.ntx);
     ProfScope p(PROF_ZB_SHADE, stream);
     // silhouettes of dense meshes are the measured case; everything else takes the full-featured variants
-    if (!rgb && !aa && !full) launch_after(4, (long long)a.B * a.R * a.R, k_zb_shade<false, false, false>, dim3(tiles), dim3(TILE_THREADS), 0, stream, a);
+    if (a.flags & FLAG_FACE_TEX) {     // per-face texture cubes (colour)
+        if (aa) launch_after(4, (long long)a.B * a.R * a.R, k_zb_shade<true, true, true, TEX_CUBE>, dim3(tiles), dim3(TILE_THREADS), 0, stream, a);
+        else launch_after(4, (long long)a.B * a.R * a.R, k_zb_shade<true, false, true, TEX_CUBE>, dim3(tiles), dim3(TILE_THREADS), 0, stream, a);
+    } else if (!rgb && !aa && !full) launch_after(4, (long long)a.B * a.R * a.R, k_zb_shade<false, false, false>, dim3(tiles), dim3(TILE_THREADS), 0, stream, a);
     else if (rgb && aa) launch_after(4, (long long)a.B * a.R * a.R, k_zb_shade<true, true, true>, dim3(tiles), dim3(TILE_THREADS), 0, stream, a);
     else if (rgb) launch_after(4, (long long)a.B * a.R * a.R, k_zb_shade<true, false, true>, dim3(tiles), dim3(TILE_THREADS), 0, stream, a);
     else if (aa) launch_after(4, (long long)a.B * a.R * a.R, k_zb_shade<false, true, true>, dim3(tiles), dim3(TILE_THREADS), 0, stream, a);

@@ -69,6 +69,35 @@ __device__ __forceinline__ void sample_texture(const float *__restrict__ tex_b, 
     }
 }
 
+// Trilinear sample of a face's own ts^3 texture cube (NR_FACE_TEXTURES; the v1 renderer's texture format).
+// cube = textures[b, face] (ts^3 texels of 3 floats, contiguous), q = weight map, z = face depths.  Tap
+// c = (c0 c1 c2) of the 8 reads texel (i_0 + c0, i_1 + c1, i_2 + c2) with weight prod_k (c_k ? f_k : 1 - f_k);
+// a tap with an index >= ts (ts = 1, or eps = 0) reads as zero.
+__device__ __forceinline__ void sample_face_texture(const float *__restrict__ cube, int ts, float eps, const float q[3],
+                                                    const float z[3], float rgb[3]) {
+    const CubeCoord cc = cube_coord(q, z, ts, eps);
+    int i[3];
+    float f[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const float fl = floorf(cc.t[k]);
+        i[k] = (int)fl;
+        f[k] = __fsub_rn(cc.t[k], fl);
+    }
+    rgb[0] = rgb[1] = rgb[2] = 0.f;
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+        const int c0 = c >> 2, c1 = (c >> 1) & 1, c2 = c & 1;
+        const int j0 = i[0] + c0, j1 = i[1] + c1, j2 = i[2] + c2;
+        if (j0 >= ts || j1 >= ts || j2 >= ts) continue;
+        const float w = __fmul_rn(__fmul_rn(c0 ? f[0] : __fsub_rn(1.f, f[0]), c1 ? f[1] : __fsub_rn(1.f, f[1])),
+                                  c2 ? f[2] : __fsub_rn(1.f, f[2]));
+        const float *p = cube + ((j0 * ts + j1) * ts + j2) * 3;
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) rgb[ch] = __fadd_rn(rgb[ch], __fmul_rn(w, __ldg(p + ch)));
+    }
+}
+
 // ---- output initialisation, done by the raster kernel itself --------------------------------------
 // The raster kernel is instruction-issue bound and leaves HBM idle, so everything that is a plain
 // fill rides along in it instead of running in front of it: the pixels of EMPTY tiles (face index -1,
@@ -224,7 +253,8 @@ __device__ __forceinline__ void do_fill_item(const RasterArgs &a, const FillPlan
 // numerators at this pixel, (bz0..2) its corner depths.  Fuses rasterize_cuda_kernel.cu:246-308 (weight map),
 // rasterize.py:100-153 (texture sampling), :252-283 (lights), :240-242 (silhouettes), :80-88 (depth),
 // :295-310 (channel merge), :315-316 (permute + flip), :321-328 (2x2 anti-aliasing mean).
-template <bool RGB, bool AA, bool FULL>
+// TEX: UV textures, or per-face cubes (FULL variants only; sample_face_texture, no aux map).
+template <bool RGB, bool AA, bool FULL, int TEX = TEX_UV>
 __device__ __forceinline__ void shade_block(const RasterArgs &a, int b, int xi, int yi, bool valid, int best,
                                             float bw0, float bw1, float bw2, float bz0, float bz1, float bz2,
                                             bool has_bg) {
@@ -299,6 +329,12 @@ __device__ __forceinline__ void shade_block(const RasterArgs &a, int b, int xi, 
         if (RGB) {
             float rgb[3] = {0.f, 0.f, 0.f};
             if (fg) {
+                if constexpr (TEX == TEX_CUBE) {
+                    // textures[b, best]: 32-bit offsets inside a view (nf ts^3 3 < 2^31, checked by the C ABI)
+                    const float z[3] = {bz0, bz1, bz2};
+                    const int ts = a.H, cube = ts * ts * ts * 3;
+                    sample_face_texture(a.tex + (size_t)b * a.nf * cube + best * cube, ts, a.eps, q, z, rgb);
+                } else {
                 // (per-view faces_textures: the launchers send those calls to the FULL variants)
                 const int32_t *fti = a.ft + (FULL ? (size_t)b * a.face_stride : 0) + 3 * (size_t)best;
                 const float *vtb = a.vt + (size_t)b * a.nvt * 2;
@@ -325,6 +361,7 @@ __device__ __forceinline__ void shade_block(const RasterArgs &a, int b, int xi, 
                     reinterpret_cast<float2 *>(aux)[1] = make_float2(q[2], tc.depth);
                     reinterpret_cast<float2 *>(aux)[2] = make_float2(tc.nx, tc.ny);
                 }
+                }   // TEX_UV
                 if (FULL && a.lights.num > 0) {
                     // smooth normal map (rasterize.py:186-187) and light accumulation (:252-283)
                     float n[3] = {0.f, 0.f, 0.f}, cw[3];

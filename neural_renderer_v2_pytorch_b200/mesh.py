@@ -1,10 +1,12 @@
 """``Mesh`` (reference ``neural_renderer_torch/mesh.py:8-37``): an ``nn.Module`` holding the vertices
-of an .obj file and a learnable legacy (v1, 6-D) texture tensor.
+of an .obj file and a learnable legacy (v1, 6-D) texture tensor: one ``ts^3`` RGB cube per face.
 
-Outside the accelerated path (SURVEY.md section 2, row 11: half-ported and unused by the reference's
-own examples); provided so that ``import neural_renderer_v2_pytorch_b200 as neural_renderer_torch``
-finds the name.  Differences: ``faces`` is kept as a tensor (the reference calls ``.expand`` on a numpy
-array, mesh.py:31) and ``to()`` returns the module."""
+The reference leaves it half-ported (SURVEY.md section 2, row 11): nothing there renders its textures.
+Here the three tensors of ``get_batch(B)`` render and differentiate as they are: faces ``[B, nf, 3]`` are
+per-view meshes, and textures ``[B, nf, ts, ts, ts, 3]`` with ``None`` for both uv inputs select the
+per-face texture cubes of the fused kernels (DESIGN.md "API notes"), e.g.
+``renderer.render(v, f, None, None, t)``.  Differences: ``faces`` is kept as a tensor (the reference calls
+``.expand`` on a numpy array, mesh.py:31) and ``to()`` returns the module."""
 import torch
 import torch.nn as nn
 

@@ -346,7 +346,8 @@ class _Rasterize(torch.autograd.Function):
         images, internal, fim, _, _, tile_list, aux = _forward_call(cfg, v, faces, vt, faces_textures, tex, False, lights, bg,
                                                                     ctx.grad_bufs or (),
                                                                     sparse=not (bg is not None and need[4]),
-                                                                    want_aux=USE_AUX_MAP and ctx.grad_bufs is not None)
+                                                                    want_aux=(USE_AUX_MAP and ctx.grad_bufs is not None and
+                                                                              not (cfg.flags & _lib.NR_FACE_TEXTURES)))
         ctx.cfg = cfg
         ctx.bg_dtype = backgrounds.dtype if backgrounds is not None else None
         ctx.has_tex = tex is not None
@@ -423,6 +424,15 @@ def _prepare(vertices, faces, params, hyperparams):
     assert faces.ndim in (2, 3)
     assert faces.shape[-1] == 3
     assert faces.ndim == 2 or faces.shape[0] == vertices.shape[0]
+    # Per-face texture cubes [B, nf, ts, ts, ts, 3] with no uv inputs (NR_FACE_TEXTURES, the textures of
+    # Mesh.get_batch, DESIGN.md "API notes"): face f of view b samples textures[b, f].
+    face_textures = bool(hyperparams.draw_rgb) and getattr(params.textures, "ndim", 0) == 6
+    if face_textures:
+        assert params.vertices_textures is None
+        assert params.faces_textures is None
+        ts = params.textures.shape[2]
+        assert ts >= 1
+        assert tuple(params.textures.shape) == (vertices.shape[0], faces.shape[-2], ts, ts, ts, 3)
     dev = vertices.device
     bg = None
     if hyperparams.draw_rgb:
@@ -449,7 +459,11 @@ def _prepare(vertices, faces, params, hyperparams):
     view_faces = faces_d.ndim == 3
     vt = ft = tex = None
     nvt = H = W = 0
-    if hyperparams.draw_rgb:
+    if face_textures:
+        tex = params.textures
+        _require_cuda(tex, "textures")
+        H = W = tex.shape[2]
+    elif hyperparams.draw_rgb:
         assert params.vertices_textures.ndim == 3
         assert params.vertices_textures.shape[2] == 2
         assert params.faces_textures.ndim in (2, 3)
@@ -472,7 +486,8 @@ def _prepare(vertices, faces, params, hyperparams):
         # the kernels read row b of both index tensors for view b: the shared one is expanded (12 B nf bytes)
         faces_d = faces_d.expand(B, nf, 3).contiguous()
     cfg = _make_config(B, nv, nf, int(hyperparams.image_size),
-                       _flags_of(hyperparams) | (_lib.NR_VIEW_FACES if view_faces else 0), hyperparams, nvt, H, W)
+                       _flags_of(hyperparams) | (_lib.NR_VIEW_FACES if view_faces else 0) |
+                       (_lib.NR_FACE_TEXTURES if face_textures else 0), hyperparams, nvt, H, W)
     light_pack = vn = None
     if hyperparams.draw_rgb and params.lights is not None:      # an empty list renders black, rasterize.py:252-283
         # shading: per-vertex normals by differentiable torch ops (O(nv + nf)), the per-pixel part in the kernels
